@@ -19,6 +19,11 @@ metric with pinned host inputs copied H2D and the logits read back D2H inside th
 occdepth_b200.serving.FramePipeline (copies on their own streams, double-buffered); the back-to-back figure is listed
 beside it.  Prints ONE JSON line (rank 0) on the original stdout; everything else this process or its libraries print
 goes to stderr.
+
+`--dump-outputs DIR` writes, after the timed steps, the outputs of the last timed forward (rank 0) as DIR/<name>.npy,
+float32: an output of up to n elements whole, a larger one as its elements at a fixed seeded set of n flat indices,
+where n = min(DUMP_MAX_ELEMS, DUMP_BUDGET_ELEMS / number of outputs) keeps the dump under 64 MB.  The inputs and weights are seeded, so two builds run with the same arguments can be
+compared output for output (`--impl reference` dumps the CPU oracle's outputs the same way).
 """
 import argparse
 import json
@@ -40,6 +45,8 @@ WORKLOAD = ("configs[1]: 1370x376 stereo, tf_efficientnet_b7_ns, flosp lift to 1
 # stated parity of the two arithmetic modes vs the CPU fp32 oracle at this configuration (tests/test_gpu_config2.py,
 # profiles/r02_config2_parity_*.json): max-abs logit diff relative to max |logit|, arg-max agreement
 TOLERANCE = {"tf32": {"rel": 1.5e-3, "argmax": 0.9984}, "bf16": {"rel": 1.4e-2, "argmax": 0.984}}
+DUMP_MAX_ELEMS = 1 << 21          # 8 MiB of float32 per dumped output
+DUMP_BUDGET_ELEMS = 15 << 20      # 60 MiB of float32 in all
 
 
 def make_cfg():
@@ -135,6 +142,22 @@ class ClockSampler(threading.Thread):
                 "samples": len(sm), "source": "nvml" if self.nvml else "nvidia-smi"}
 
 
+def dump_outputs(out, directory):
+    """write each tensor of the forward's output dict as <directory>/<name>.npy (float32), sampled as the module
+    docstring describes"""
+    import numpy as np
+    import torch
+    os.makedirs(directory, exist_ok=True)
+    tensors = {k: v for k, v in out.items() if isinstance(v, torch.Tensor)}
+    n = min(DUMP_MAX_ELEMS, DUMP_BUDGET_ELEMS // max(1, len(tensors)))
+    for name, t in sorted(tensors.items()):
+        flat = t.detach().float().flatten()
+        if flat.numel() > n:
+            idx = np.sort(np.random.default_rng(0).choice(flat.numel(), n, replace=False))
+            flat = flat[torch.from_numpy(idx).to(flat.device)]
+        np.save(os.path.join(directory, name + ".npy"), flat.cpu().numpy())
+
+
 def oracle_inputs(device=None):
     """state dict + batch + cfg of the workload for oracle/functional.py (the reference algorithm)"""
     m = build_model()
@@ -171,10 +194,11 @@ def cpu_forward_seconds(steps=1, warmup=0):
     with torch.no_grad():
         for i in range(warmup + steps):
             t0 = time.perf_counter()
-            OF.occdepth_forward(sd, batch, cfg)
+            out = OF.occdepth_forward(sd, batch, cfg)
             dt = time.perf_counter() - t0
             if i >= warmup:
                 times.append(dt)
+    cpu_forward_seconds.last_output = out
     return times, torch.get_num_threads()
 
 
@@ -183,6 +207,8 @@ def run_reference(args):
     if rank != 0:
         return
     times, cores = cpu_forward_seconds(args.steps, args.warmup)
+    if args.dump_outputs:
+        dump_outputs(cpu_forward_seconds.last_output, args.dump_outputs)
     total = sum(times)
     v = N_OUT * len(times) / total
     line = {
@@ -328,6 +354,8 @@ def run_b200(args):
         reps.append((ms_r, dict(time_forwards.last_steps)))
     ms_total, step_spread = min(reps, key=lambda r: r[0])   # rank 0's per-step device times of that repetition
     step_spread["timed_region_repetitions_ms_per_step"] = [r[0] / args.steps for r in reps]
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(out, args.dump_outputs)
 
     # ---- end-to-end arm: host buffers, H2D of the inputs and D2H of the logits inside the timed region ----
     img_h, pix_h, fov_h = img.pin_memory(), pix.pin_memory(), fov.pin_memory()
@@ -691,6 +719,8 @@ def main():
                     help="frames: one frame per GPU (default, weak scaling; N > 1 adds a `slab` block); slab: the "
                          "X-slab partition of one frame as the headline")
     ap.add_argument("--dump-profile", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed forward's outputs to DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
     if args.impl == "reference":
         return run_reference(args)

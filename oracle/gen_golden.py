@@ -1,11 +1,16 @@
-"""Generates tests/golden/*.pt by running the UNMODIFIED reference (imported from /root/reference through
-oracle/ref_import.py) on seeded inputs and weights.  Run in the build container:  python -m oracle.gen_golden
+"""Generates tests/golden/* by running the UNMODIFIED reference (imported through oracle/ref_import.py, which finds
+its source tree through OCCDEPTH_REFERENCE) on seeded inputs and weights:  python -m oracle.gen_golden
 
 Each fixture stores the inputs (or the seed that regenerates them), the seed of `synth.seed_weights_`, and the
 reference outputs (fp16-safe small tensors kept as fp32).
 """
+import copy
+import hashlib
+import json
+import lzma
 import os
 
+import numpy as np
 import torch
 import torch.nn as nn
 
@@ -105,11 +110,131 @@ def gen_vox2pix():
     out = {}
     for name, E, K, org, vs, W, H, scene, pid in vox2pix_cases():
         pix, fov, z = helpers.vox2pix(E, K, org, vs, W, H, scene, pid)
+        if np.array_equal(pix.astype(np.int16), pix):      # stored as int16 where that is lossless (file size)
+            pix = pix.astype(np.int16)
         out[name] = dict(cam_E=torch.from_numpy(E.copy()), cam_k=torch.from_numpy(K.copy()),
                          vox_origin=torch.from_numpy(org.copy()), voxel_size=vs, img_W=W, img_H=H,
                          scene_size=scene, pattern_id=pid, pix=torch.from_numpy(pix), fov=torch.from_numpy(fov),
                          pix_z=torch.from_numpy(z))
     torch.save(out, os.path.join(OUT, "vox2pix.pt"))
+
+
+def pack(t, full_max=1024):
+    """a reference output for the golden file: all of it up to `full_max` elements, else its elements at
+    reference_cases.sample_index; with the float64 sum and absolute sum of the whole tensor"""
+    from .reference_cases import sample_index
+    t = t.detach().float().contiguous()
+    flat = t.flatten()
+    d = dict(shape=tuple(t.shape), sum=float(t.double().sum()), abs_sum=float(t.double().abs().sum()),
+             sampled=flat.numel() > full_max)
+    d["values"] = flat[sample_index(flat.numel())].clone() if d["sampled"] else flat.clone()
+    return d
+
+
+def array_digest(a):
+    """sha256 of an array's dtype, shape and bytes (NaNs canonicalised): bit-exact comparisons without the array"""
+    a = np.array(a)
+    if a.dtype.kind == "f":
+        a[np.isnan(a)] = np.nan
+    h = hashlib.sha256(("%s%s" % (a.dtype.str, a.shape)).encode())
+    h.update(np.ascontiguousarray(a).tobytes())
+    return h.hexdigest()
+
+
+def gen_reference_outputs():
+    """what tests/test_oracle_vs_reference.py compares the oracle with: the reference modules' outputs on the seeded
+    cases of oracle/reference_cases.py, and digests of the numba vox2pix for every case and pattern"""
+    from . import reference_cases as RC
+    ns = RC.reference_modules()
+    out = {}
+    with torch.no_grad():
+        for ds, V, P in RC.SFA_CASES:
+            c = RC.sfa(ds, V, P)
+            y = ns.SFA.SFA(c["scene"], ds, c["ps"])(c["x2d"], c["pix"].clone(), c["fov"].clone())
+            out["sfa[%s-%d-%d]" % (ds, V, P)] = dict(out=pack(y.contiguous()))
+        proc, down, up, x = RC.bottleneck(ns)
+        y = down(x)
+        out["bottleneck"] = dict(state_sum=RC.state_sum(proc, down, up), process=pack(proc(x)),
+                                 downsample=pack(y, full_max=y.numel()), upsample=pack(up(y)))
+        for which in ("kitti", "nyu"):
+            m, x = RC.unet3d(ns, which)
+            out["unet3d[%s]" % which] = dict(state_sum=RC.state_sum(m),
+                                             out={k: pack(v) for k, v in m({"x3d": x}).items()})
+        m, x = RC.unet2d(ns)
+        out["unet2d"] = dict(state_sum=RC.state_sum(m), out={k: pack(v) for k, v in m(x).items()})
+        m, batch, _ = RC.occdepth_small(ns)
+        out["occdepth_small"] = dict(state_sum=RC.state_sum(m), out={k: pack(v) for k, v in m(batch).items()})
+        m, _, args = RC.flosp_depth(ns)
+        y, d = m(*args, None)
+        out["flosp_depth"] = dict(state_sum=RC.state_sum(m), out=pack(y), depth=pack(d),
+                                  covered=float((y > 0).float().mean()))
+        m, batch, _ = RC.occdepth_nyu_virtual_view(ns)
+        out["occdepth_nyu_virtual_view"] = dict(state_sum=RC.state_sum(m),
+                                                out={k: pack(v) for k, v in m(batch).items()})
+    helpers = ref_import.data_helpers()
+    for pid in RC.VOX2PIX_PATTERNS:
+        for name, E, K, org, vs, W, H, scene, _ in vox2pix_cases():
+            out["vox2pix[%s-%d]" % (name, pid)] = [array_digest(a) for a in helpers.vox2pix(E, K, org, vs, W, H,
+                                                                                              scene, pid)]
+    torch.save(out, os.path.join(OUT, "reference_outputs.pt"))
+
+
+def gen_state_dict_keys():
+    """state_dict layout (key, shape, dtype) of the reference modules in the configurations of
+    tests/test_state_dict_compat.py, and the reference's FlospDepth configuration map"""
+    from . import reference_cases as RC
+    ns = RC.reference_modules()
+
+    def layout(m):
+        return [[k, list(v.shape), str(v.dtype)] for k, v in m.state_dict().items()]
+    out = {}
+    with ref_import.quiet():
+        for name, args, kw in state_dict_configs():
+            if name.startswith("unet3d_kitti"):
+                out[name] = layout(ns.unet3d_kitti.UNet3D(*args, **kw))
+            elif name.startswith("unet3d_nyu"):
+                out[name] = layout(ns.unet3d_nyu.UNet3D(*args, **kw))
+            elif name.startswith("unet2d"):
+                out[name] = layout(ns.unet2d.UNet2D.build(**kw))
+            elif name.startswith("flosp_depth"):
+                c = copy.deepcopy(ns.flosp_depth_conf_map[kw["dataset"]])
+                c.update(kw["update"])
+                out[name] = layout(ns.FlospDepth(**c))
+            else:
+                cfg = synth.Cfg(kw)
+                saved = copy.deepcopy(ns.flosp_depth_conf_map)
+                try:
+                    out[name] = layout(ns.OccDepth.OccDepth(["c"] * cfg.n_classes, torch.ones(cfg.n_classes),
+                                                            full_scene_size=cfg.full_scene_size,
+                                                            project_res=RC.PROJECT_RES, config=cfg))
+                finally:       # the reference mutates the module-level conf dicts in place (OccDepth.py:183-198)
+                    for k, v in saved.items():
+                        ns.flosp_depth_conf_map[k].clear()
+                        ns.flosp_depth_conf_map[k].update(v)
+    out["flosp_depth_conf_map"] = json.loads(json.dumps(ns.flosp_depth_conf_map))
+    with lzma.open(os.path.join(OUT, "state_dict_keys.json.xz"), "wt") as f:
+        json.dump(out, f, separators=(",", ":"))
+
+
+def state_dict_configs():
+    """(name, args, kwargs) of every module configuration whose state_dict layout tests/test_state_dict_compat.py
+    checks; OccDepth entries carry their config dict as kwargs"""
+    k3 = dict(context_prior=True, cascade_cls=True, occluded_cls=True)
+    cfgs = [("unet3d_kitti[full]", (20, nn.BatchNorm3d, (256, 256, 32), 64, 2), k3),
+            ("unet3d_nyu[full]", (12, nn.BatchNorm3d, 200, (60, 36, 60)), {}),
+            ("unet3d_kitti[project_scale_1]", (20, nn.BatchNorm3d, (128, 128, 16), 32, 1), {})]
+    for b in ("tf_efficientnet_b3_ns", "tf_efficientnet_b4_ns", "tf_efficientnet_b5_ns", "tf_efficientnet_b7_ns"):
+        cfgs.append(("unet2d[%s]" % b, (), dict(out_feature=64, use_decoder=True, backbone_2d_name=b,
+                                                 return_up_feats=1)))
+    for ds, scene, ps in (("kitti", (256, 256, 32), 2), ("NYU", (60, 36, 60), 1)):
+        cfgs.append(("flosp_depth[%s]" % ds, (), dict(dataset=ds, update=dict(scene_size=scene, project_scale=ps,
+                                                                              return_depth=False))))
+    cfgs.append(("occdepth[kitti_flosp]", (), dict(synth.occdepth_cfg(trans_2d_to_3d="flosp"))))
+    cfgs.append(("occdepth[kitti_flosp_depth]", (), dict(synth.occdepth_cfg(trans_2d_to_3d="flosp_depth"))))
+    cfgs.append(("occdepth[nyu_flosp]", (), dict(synth.occdepth_cfg(
+        dataset="NYU", full_scene_size=(60, 36, 60), project_scale=1, feature=200, feature_2d_oc=200, n_classes=12,
+        cascade_cls=False))))
+    return cfgs
 
 
 def main():
@@ -120,6 +245,8 @@ def main():
     gen_unet3d(ref)
     gen_occdepth(ref)
     gen_vox2pix()
+    gen_reference_outputs()
+    gen_state_dict_keys()
     for f in sorted(os.listdir(OUT)):
         print(f, os.path.getsize(os.path.join(OUT, f)))
 

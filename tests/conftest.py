@@ -1,8 +1,6 @@
 import os
 import sys
 
-import pytest
-
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
@@ -10,16 +8,9 @@ if ROOT not in sys.path:
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (B200); run with -m gpu on the GPU box")
-    config.addinivalue_line("markers", "reference: needs the reference tree at /root/reference (build container only)")
 
 
 def pytest_collection_modifyitems(config, items):
-    from oracle import ref_import
-    have_ref = ref_import.available()
-    skip_ref = pytest.mark.skip(reason="reference tree (/root/reference) not present on this machine")
-    for item in items:
-        if "reference" in item.keywords and not have_ref:
-            item.add_marker(skip_ref)
     # kernel-level GPU tests first: a broken kernel fails in seconds, before the full-size model tests spend minutes
     # on CPU oracle forwards -- and the process's first launches are the library's own tcgen05 kernels
     order = ["test_gpu_conv", "test_gpu_ops", "test_gpu_sfa", "test_gpu_unet3d", "test_gpu_net2d", "test_gpu_golden",

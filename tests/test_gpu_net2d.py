@@ -165,7 +165,7 @@ def test_occdepth_forward_flosp_depth(precision):
 def test_occdepth_forward_nyu_virtual_view(precision):
     """config-4-type path: single RGB view + gt_depth -> virtual right view kernel -> lift -> NYU 3D net"""
     from occdepth_b200.models.OccDepth import OccDepth
-    from test_oracle_vs_reference import _nyu_virtual_batch
+    from oracle.reference_cases import nyu_virtual_batch
     torch.manual_seed(0)
     full = (12, 8, 12)
     cfg = synth.occdepth_cfg(dataset="NYU", full_scene_size=full, project_scale=1, feature=16, feature_2d_oc=16,
@@ -174,7 +174,7 @@ def test_occdepth_forward_nyu_virtual_view(precision):
         m = OccDepth(["c"] * 6, torch.ones(6), full_scene_size=full, project_res=["1", "2", "4", "8"],
                      config=cfg).eval()
     synth.seed_weights_(m, 3)
-    batch = _nyu_virtual_batch(32, 64, full)
+    batch = nyu_virtual_batch(32, 64, full)
     ocfg = dict(cfg)
     ocfg["project_res"] = ["1", "2", "4", "8"]
     with torch.no_grad():
