@@ -11,7 +11,6 @@
 #include "conv_common.cuh"
 #include "conv_tc.cuh"
 #include <new>
-#include <utility>
 #include <stdio.h>
 #include <string.h>
 #include <stdlib.h>
@@ -19,7 +18,89 @@
 namespace {
 
 constexpr int kTcThreads = 576;  // warp 0: TMA producer, warp 1: MMA issuer (+TMEM alloc), warps 2-17: four epilogue groups
-constexpr int kMaxStages = 24;
+constexpr int kMaxStages = 24;   // smem ring stages of the per-tap kernel
+constexpr int kHaloMaxStages = 4;
+
+// mbarriers of a persistent tcgen05 conv CTA, placed after its operand buffers: full[max_stages], empty[max_stages],
+// two TMEM accumulator pairs tfull[2] / tempty[2], the resident-weight barrier w (halo kernels), and the 4-byte slot
+// tcgen05.alloc writes the TMEM base address to
+struct CtaBarriers {
+  uint32_t full, empty, tfull, tempty, w, slot;
+};
+
+__device__ __forceinline__ CtaBarriers cta_barriers(uint32_t base, int max_stages) {
+  CtaBarriers b;
+  b.full = base;
+  b.empty = base + 8u * max_stages;
+  b.tfull = base + 16u * max_stages;
+  b.tempty = b.tfull + 16u;
+  b.w = b.tempty + 16u;
+  b.slot = b.w + 8u;
+  return b;
+}
+
+// Prologue of the three persistent kernels: tensor-map prefetch and barrier init (thread 0), TMEM alloc (warp 1),
+// then the wait for the previous grid (programmatic dependent launch, common.cuh; without it griddepcontrol.wait
+// returns at once).  Everything before the wait overlaps the tail of the previous grid, whose results are only
+// touched after it.  Returns the TMEM base address.
+__device__ __forceinline__ uint32_t cta_prologue(const CtaBarriers& bar, int stages, bool w_bar, int tmem_cols,
+                                                 const CUtensorMap* tmA, const CUtensorMap* tmW) {
+  if (threadIdx.x == 0) {
+    tc::prefetch_tmap(tmA);
+    tc::prefetch_tmap(tmW);
+    for (int s = 0; s < stages; ++s) {
+      tc::mbar_init(bar.full + 8u * s, 1);
+      tc::mbar_init(bar.empty + 8u * s, 1);
+    }
+    for (int a = 0; a < 2; ++a) {
+      tc::mbar_init(bar.tfull + 8u * a, 1);
+      tc::mbar_init(bar.tempty + 8u * a, 256);  // every epilogue thread of the two groups arrives
+    }
+    if (w_bar) tc::mbar_init(bar.w, 1);
+    tc::fence_barrier_init();
+  }
+  if ((threadIdx.x >> 5) == 1) {
+    __syncwarp();
+    tc::tmem_alloc(bar.slot, (uint32_t)tmem_cols);
+  }
+  tc::fence_before_sync();
+  __syncthreads();
+  tc::fence_after_sync();
+  uint32_t tmem_base;
+  asm volatile("ld.shared.b32 %0, [%1];" : "=r"(tmem_base) : "r"(bar.slot));
+  asm volatile("griddepcontrol.wait;" ::: "memory");
+  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
+  return tmem_base;
+}
+
+__device__ __forceinline__ void cta_teardown(uint32_t tmem_base, int tmem_cols) {
+  tc::fence_before_sync();
+  __syncthreads();
+  if ((threadIdx.x >> 5) == 1) {
+    __syncwarp();
+    tc::tmem_dealloc(tmem_base, (uint32_t)tmem_cols);
+  }
+}
+
+// Debug timeline (occd_conv_debug_trace, tools/conv_trace.py): clock64 stamp k of pipeline step j of CTA 0 into
+// trace[64][8].  k = 0 / 1: TMA producer, 2 / 3: MMA issuer, 4 / 5 / 6: epilogue wait / go / done (thread 64 only)
+__device__ __forceinline__ void trace_stamp(long long* trace, uint32_t j, int k) {
+  if (trace && blockIdx.x == 0 && j < 64u && (k < 4 || threadIdx.x == 64)) trace[j * 8 + k] = clock64();
+}
+
+// Fast epilogue (conv_common.cuh) of this thread's accumulator row: TMEM columns [c_begin, c_end) from taddr, each
+// chunk's bias / residual loads in flight together with its TMEM load
+template <typename T>
+__device__ __forceinline__ void epi_drain_fast(const EpiRow<T>& er, uint32_t taddr, int c_begin, int c_end) {
+  uint32_t ra[16];
+  EpiPre q;
+  for (int c0 = c_begin; c0 < c_end; c0 += 16) {
+    tc::tmem_ld16_issue(taddr + (uint32_t)c0, ra);
+    epi_prefetch<T>(er, c0, q);
+    tc::tmem_ld_wait16(ra);
+    epi_finish<T>(er, c0, ra, q);
+  }
+}
 
 struct TcParams {
   ConvEpi epi;
@@ -35,7 +116,6 @@ struct TcParams {
   int stages, group;
   int a_bytes, b_stride, b_bytes;
   int tmem_cols;
-  int pdl;           // launched with programmatic stream serialization: wait for the producer grid after the prologue
   long long* trace;  // optional [tile][8] clock64 stamps of CTA 0 (occd_conv_debug_trace, tools/conv_trace.py)
   signed char tap_src[OCCD_CONV_MAX_TAPS];
   short tap_dz[OCCD_CONV_MAX_TAPS], tap_dy[OCCD_CONV_MAX_TAPS], tap_dx[OCCD_CONV_MAX_TAPS];
@@ -72,12 +152,8 @@ conv_tc_kernel(const __grid_constant__ TcParams p, const __grid_constant__ CUten
   const uint32_t smem_base = (tc::smem_u32(smem_raw) + 1023u) & ~1023u;
   const uint32_t smem_a = smem_base;
   const uint32_t smem_b = smem_a + (uint32_t)(p.stages * p.group) * p.a_bytes;
-  const uint32_t bar_base = smem_b + (uint32_t)(p.stages * p.group) * p.b_stride;  // 8-byte aligned (multiples of 1024)
-  const uint32_t full_bar = bar_base;
-  const uint32_t empty_bar = bar_base + 8u * kMaxStages;
-  const uint32_t tmem_full_bar = bar_base + 16u * kMaxStages;       // [2]
-  const uint32_t tmem_empty_bar = tmem_full_bar + 16u;              // [2]
-  const uint32_t tmem_slot = tmem_empty_bar + 16u;
+  // barriers: 8-byte aligned (the buffers before them are multiples of 1024 bytes)
+  const CtaBarriers bar = cta_barriers(smem_b + (uint32_t)(p.stages * p.group) * p.b_stride, kMaxStages);
 
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
@@ -85,34 +161,7 @@ conv_tc_kernel(const __grid_constant__ TcParams p, const __grid_constant__ CUten
   const int tiles_per_group = p.num_m_tiles * n_tiles_n;
   const int num_tiles = tiles_per_group * p.n_groups;
 
-  if (warp == 0 && lane == 0) {
-    tc::prefetch_tmap(&tmA0);
-    tc::prefetch_tmap(&tmW);
-    for (int s = 0; s < p.stages; ++s) {
-      tc::mbar_init(full_bar + 8u * s, 1);
-      tc::mbar_init(empty_bar + 8u * s, 1);
-    }
-    for (int a = 0; a < 2; ++a) {
-      tc::mbar_init(tmem_full_bar + 8u * a, 1);
-      tc::mbar_init(tmem_empty_bar + 8u * a, 256);  // every epilogue thread of the two groups arrives
-    }
-    tc::fence_barrier_init();
-  }
-  if (warp == 1) {
-    __syncwarp();
-    tc::tmem_alloc(tmem_slot, (uint32_t)p.tmem_cols);
-  }
-  tc::fence_before_sync();
-  __syncthreads();
-  tc::fence_after_sync();
-  uint32_t tmem_base;
-  asm volatile("ld.shared.b32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot));
-  if (p.pdl) {
-    // programmatic dependent launch: everything above (barrier init, TMEM alloc, tensor-map prefetch) overlapped
-    // the tail of the producer grid; its results are only touched below this point
-    asm volatile("griddepcontrol.wait;" ::: "memory");
-    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-  }
+  const uint32_t tmem_base = cta_prologue(bar, p.stages, false, p.tmem_cols, &tmA0, &tmW);
   const uint32_t acc_stride = (uint32_t)p.tmem_cols >> 1;  // column offset of the second accumulator
 
   if (warp == 0) {
@@ -137,7 +186,7 @@ conv_tc_kernel(const __grid_constant__ TcParams p, const __grid_constant__ CUten
         int g = 0;
         int remaining = p.grp_iters[grp];
         const int jt = (tile - blockIdx.x) / gridDim.x;
-        if (p.trace && blockIdx.x == 0 && jt < 64) p.trace[jt * 8 + 0] = clock64();
+        trace_stamp(p.trace, jt, 0);
         for (int tp = p.grp_tap0[grp]; tp < p.grp_tap0[grp + 1]; ++tp) {
           const int src = p.tap_src[tp];
           const int cw = iw0 + p.tap_dx[tp], ch = ih0 + p.tap_dy[tp], cd = id0 + p.tap_dz[tp];
@@ -146,13 +195,13 @@ conv_tc_kernel(const __grid_constant__ TcParams p, const __grid_constant__ CUten
           for (int kc = 0; kc < nk; ++kc) {
             if (g == 0) {
               const int cnt = remaining < p.group ? remaining : p.group;
-              tc::mbar_wait(empty_bar + 8u * s, ph ^ 1u);
-              tc::mbar_expect_tx(full_bar + 8u * s, (uint32_t)(cnt * (p.a_bytes + p.b_bytes)));
+              tc::mbar_wait(bar.empty + 8u * s, ph ^ 1u);
+              tc::mbar_expect_tx(bar.full + 8u * s, (uint32_t)(cnt * (p.a_bytes + p.b_bytes)));
             }
             const uint32_t sa = smem_a + (uint32_t)(s * p.group + g) * p.a_bytes;
             const uint32_t sb = smem_b + (uint32_t)(s * p.group + g) * p.b_stride;
-            tc::tma_load_5d(sa, maps[src], full_bar + 8u * s, kc * KCH, cw, ch, cd, b);
-            tc::tma_load_2d(sb, &tmW, full_bar + 8u * s, kc * KCH, wrow);
+            tc::tma_load_5d(sa, maps[src], bar.full + 8u * s, kc * KCH, cw, ch, cd, b);
+            tc::tma_load_2d(sb, &tmW, bar.full + 8u * s, kc * KCH, wrow);
             --remaining;
             if (++g == p.group || remaining == 0) {
               g = 0;
@@ -160,7 +209,7 @@ conv_tc_kernel(const __grid_constant__ TcParams p, const __grid_constant__ CUten
             }
           }
         }
-        if (p.trace && blockIdx.x == 0 && jt < 64) p.trace[jt * 8 + 1] = clock64();
+        trace_stamp(p.trace, jt, 1);
       }
     }
   } else if (warp == 1) {
@@ -174,28 +223,25 @@ conv_tc_kernel(const __grid_constant__ TcParams p, const __grid_constant__ CUten
       int j = 0;
       for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x, ++j) {
         const uint32_t acc = (uint32_t)j & 1u;
-        tc::mbar_wait(tmem_empty_bar + 8u * acc, (((uint32_t)j >> 1) & 1u) ^ 1u);  // epilogue drained this buffer
+        tc::mbar_wait(bar.tempty + 8u * acc, (((uint32_t)j >> 1) & 1u) ^ 1u);  // epilogue drained this buffer
         tc::fence_after_sync();
-        if (p.trace && blockIdx.x == 0 && j < 64) p.trace[j * 8 + 2] = clock64();
+        trace_stamp(p.trace, j, 2);
         const uint32_t d_tmem = tmem_base + acc * acc_stride;
         const int iters_per_tile = p.grp_iters[tile / tiles_per_group];
         for (int it = 0; it < iters_per_tile;) {
-          tc::mbar_wait(full_bar + 8u * s, ph);
+          tc::mbar_wait(bar.full + 8u * s, ph);
           tc::fence_after_sync();
           const int cnt = (iters_per_tile - it) < p.group ? (iters_per_tile - it) : p.group;
           for (int g = 0; g < cnt; ++g, ++it) {
             const uint64_t da = da0 + (uint64_t)((s * p.group + g) * (p.a_bytes >> 4));
             const uint64_t db = db0 + (uint64_t)((s * p.group + g) * (p.b_stride >> 4));
-            if (it == 0) tc::Mma<T>::template issue<0>(d_tmem, da, db, idesc);
-            else tc::Mma<T>::template issue<1>(d_tmem, da, db, idesc);
-#pragma unroll
-            for (int k = 1; k < NMMA; ++k) tc::Mma<T>::template issue<1>(d_tmem, da + 2 * k, db + 2 * k, idesc);
+            tc::mma_kchunk<T, NMMA>(d_tmem, da, db, idesc, it == 0);
           }
-          tc::mma_commit(empty_bar + 8u * s);  // frees the smem stage when these MMAs retire
+          tc::mma_commit(bar.empty + 8u * s);  // frees the smem stage when these MMAs retire
           if (++s == p.stages) { s = 0; ph ^= 1u; }
         }
-        tc::mma_commit(tmem_full_bar + 8u * acc);  // accumulator complete
-        if (p.trace && blockIdx.x == 0 && j < 64) p.trace[j * 8 + 3] = clock64();
+        tc::mma_commit(bar.tfull + 8u * acc);  // accumulator complete
+        trace_stamp(p.trace, j, 3);
       }
     }
   } else {
@@ -215,7 +261,6 @@ conv_tc_kernel(const __grid_constant__ TcParams p, const __grid_constant__ CUten
     const int rw = row % p.TW;
     const int rh = (row / p.TW) % p.TH;
     const int rd = row / (p.TW * p.TH);
-    const bool tracer = p.trace && blockIdx.x == 0 && threadIdx.x == 64;
     int j = 0;
     for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x, ++j) {
       if ((j & 1) != grp) continue;
@@ -231,10 +276,10 @@ conv_tc_kernel(const __grid_constant__ TcParams p, const __grid_constant__ CUten
       const bool valid = od < p.epi.OD && oh < p.epi.OH && ow < p.epi.OW && (!XP || (rw >= 1 && rw <= 30));
       const int n0 = nt * p.N_tile;
       const uint32_t acc = (uint32_t)grp;
-      if (tracer && j < 64) p.trace[j * 8 + 4] = clock64();
-      tc::mbar_wait(tmem_full_bar + 8u * acc, ((uint32_t)j >> 1) & 1u);
+      trace_stamp(p.trace, j, 4);
+      tc::mbar_wait(bar.tfull + 8u * acc, ((uint32_t)j >> 1) & 1u);
       tc::fence_after_sync();
-      if (tracer && j < 64) p.trace[j * 8 + 5] = clock64();
+      trace_stamp(p.trace, j, 5);
       const uint32_t taddr = tmem_base + acc * acc_stride + ((uint32_t)(q * 32) << 16);
       if constexpr (XP) {
         // TW == 32: lane == tile column, so the W neighbours' partial sums sit in the neighbouring lanes
@@ -249,38 +294,26 @@ conv_tc_kernel(const __grid_constant__ TcParams p, const __grid_constant__ CUten
           if (valid) conv_epilogue_row<T, 16>(p.epi, b, od, oh, ow, c0, v);
         }
       } else if (epi_fast_ok(p.epi)) {
-        // fast path (conv_common.cuh): bias / residual loads ahead of the accumulator, pointers formed once per tile
+        // fast path: pointers formed once per tile
         const EpiRow<T> er = p.n_groups > 1 ? epi_row<T>(p.epi, valid, b, od, oh, ow, n0, p.grp_oadd[tgrp][0],
                                                          p.grp_oadd[tgrp][1], p.grp_oadd[tgrp][2])
                                             : epi_row<T>(p.epi, valid, b, od, oh, ow, n0);
-        uint32_t ra[16];
-        EpiPre q;
-        for (int c0 = c_begin; c0 < c_end; c0 += 16) {
-          tc::tmem_ld16_issue(taddr + (uint32_t)c0, ra);
-          epi_prefetch<T>(er, c0, q);                        // in flight together with the TMEM load of this chunk
-          tc::tmem_ld_wait16(ra);
-          epi_finish<T>(er, c0, ra, q);
-        }
+        epi_drain_fast<T>(er, taddr, c_begin, c_end);
       } else {
         // software-pipelined: the tcgen05.ld of this group's next 16 columns is in flight while these are stored
         uint32_t ra[16], rb[16];
         int c0 = c_begin;
-        long long t_ld = 0, t_epi = 0, t_a = 0;
         if (c0 < c_end) tc::tmem_ld16_issue(taddr + (uint32_t)c0, ra);
         for (; c0 < c_end; c0 += 32) {
-          if (tracer) t_a = clock64();
           tc::tmem_ld_wait16(ra);
-          if (tracer) t_ld += clock64() - t_a;
           const bool has_b = c0 + 16 < c_end;
           if (has_b) tc::tmem_ld16_issue(taddr + (uint32_t)(c0 + 16), rb);
-          if (tracer) t_a = clock64();
           if (valid) {
             float v[16];
 #pragma unroll
             for (int i = 0; i < 16; ++i) v[i] = __uint_as_float(ra[i]);
             conv_epilogue_row<T, 16>(p.epi, b, od, oh, ow, n0 + c0, v);
           }
-          if (tracer) t_epi += clock64() - t_a;
           if (has_b) {
             tc::tmem_ld_wait16(rb);
             if (c0 + 32 < c_end) tc::tmem_ld16_issue(taddr + (uint32_t)(c0 + 32), ra);
@@ -292,19 +325,13 @@ conv_tc_kernel(const __grid_constant__ TcParams p, const __grid_constant__ CUten
             }
           }
         }
-        if (tracer && j < 64) p.trace[j * 8 + 7] = (t_ld << 32) | (t_epi & 0xffffffffll);
       }
       tc::fence_before_sync();
-      tc::mbar_arrive(tmem_empty_bar + 8u * acc);  // this thread's TMEM reads of the buffer are done
-      if (tracer && j < 64) p.trace[j * 8 + 6] = clock64();
+      tc::mbar_arrive(bar.tempty + 8u * acc);  // this thread's TMEM reads of the buffer are done
+      trace_stamp(p.trace, j, 6);
     }
   }
-  tc::fence_before_sync();
-  __syncthreads();
-  if (warp == 1) {
-    __syncwarp();
-    tc::tmem_dealloc(tmem_base, (uint32_t)p.tmem_cols);
-  }
+  cta_teardown(tmem_base, p.tmem_cols);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -334,7 +361,6 @@ struct HaloParams {
   int N_tile, tmem_cols, set_stride;
   int b_stride, w_bytes;
   int tap_off16[27];          // (R0 + (a*PH + b)*PW + c) * row_bytes / 16: A-descriptor advance per tap
-  int pdl;                    // see TcParams::pdl
   long long* trace;
 };
 
@@ -347,13 +373,7 @@ conv_halo_kernel(const __grid_constant__ HaloParams p, const __grid_constant__ C
   const uint32_t smem_base = (tc::smem_u32(smem_raw) + 1023u) & ~1023u;
   const uint32_t smem_w = smem_base;                                   // [n_taps][b_stride] resident weights
   const uint32_t smem_a = smem_w + (uint32_t)p.w_bytes;                 // [stages][a_stage_bytes]
-  const uint32_t bar_base = smem_a + (uint32_t)p.stages * p.a_stage_bytes;
-  const uint32_t full_bar = bar_base;            // [4]
-  const uint32_t empty_bar = bar_base + 32u;     // [4]
-  const uint32_t tfull_bar = bar_base + 64u;     // [2]
-  const uint32_t tempty_bar = bar_base + 80u;    // [2]
-  const uint32_t w_bar = bar_base + 96u;
-  const uint32_t tmem_slot = bar_base + 104u;
+  const CtaBarriers bar = cta_barriers(smem_a + (uint32_t)p.stages * p.a_stage_bytes, kHaloMaxStages);
 
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
@@ -361,33 +381,7 @@ conv_halo_kernel(const __grid_constant__ HaloParams p, const __grid_constant__ C
   const int per_res = p.tilesD * p.tilesH * p.tilesW;
   const int num_tiles = p.epi.B * d * d * d * per_res;
 
-  if (warp == 0 && lane == 0) {
-    tc::prefetch_tmap(&tmA);
-    tc::prefetch_tmap(&tmW);
-    for (int s = 0; s < p.stages; ++s) {
-      tc::mbar_init(full_bar + 8u * s, 1);
-      tc::mbar_init(empty_bar + 8u * s, 1);
-    }
-    for (int a = 0; a < 2; ++a) {
-      tc::mbar_init(tfull_bar + 8u * a, 1);
-      tc::mbar_init(tempty_bar + 8u * a, 256);
-    }
-    tc::mbar_init(w_bar, 1);
-    tc::fence_barrier_init();
-  }
-  if (warp == 1) {
-    __syncwarp();
-    tc::tmem_alloc(tmem_slot, (uint32_t)p.tmem_cols);
-  }
-  tc::fence_before_sync();
-  __syncthreads();
-  tc::fence_after_sync();
-  uint32_t tmem_base;
-  asm volatile("ld.shared.b32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot));
-  if (p.pdl) {
-    asm volatile("griddepcontrol.wait;" ::: "memory");
-    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-  }
+  const uint32_t tmem_base = cta_prologue(bar, p.stages, true, p.tmem_cols, &tmA, &tmW);
 
   // tile -> (batch, residue class, sub-grid tile origin)
   auto decode = [&](int tile, int& b, int& ra, int& rb, int& rc, int& td, int& th, int& tw) {
@@ -404,17 +398,17 @@ conv_halo_kernel(const __grid_constant__ HaloParams p, const __grid_constant__ C
   if (warp == 0) {
     if (lane == 0) {
       // ===== TMA producer: resident weights once, then one halo box per tile =====
-      tc::mbar_expect_tx(w_bar, (uint32_t)(p.n_taps * p.N_tile * RB));
+      tc::mbar_expect_tx(bar.w, (uint32_t)(p.n_taps * p.N_tile * RB));
       for (int tp = 0; tp < p.n_taps; ++tp)
-        tc::tma_load_2d(smem_w + (uint32_t)tp * p.b_stride, &tmW, w_bar, 0, tp * p.N_tile);
+        tc::tma_load_2d(smem_w + (uint32_t)tp * p.b_stride, &tmW, bar.w, 0, tp * p.N_tile);
       int s = 0;
       uint32_t ph = 0;
       for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
         int b, ra, rb, rc, td, th, tw;
         decode(tile, b, ra, rb, rc, td, th, tw);
-        tc::mbar_wait(empty_bar + 8u * s, ph ^ 1u);
-        tc::mbar_expect_tx(full_bar + 8u * s, (uint32_t)p.box_bytes);
-        tc::tma_load_5d(smem_a + (uint32_t)s * p.a_stage_bytes, &tmA, full_bar + 8u * s, 0,
+        tc::mbar_wait(bar.empty + 8u * s, ph ^ 1u);
+        tc::mbar_expect_tx(bar.full + 8u * s, (uint32_t)p.box_bytes);
+        tc::tma_load_5d(smem_a + (uint32_t)s * p.a_stage_bytes, &tmA, bar.full + 8u * s, 0,
                         (tw * p.BW - p.hw) * d + rc, (th * p.BH - p.hh) * d + rb,
                         (td * p.BD - p.hd) * d + ra + p.src_d0, b);
         if (++s == p.stages) { s = 0; ph ^= 1u; }
@@ -426,40 +420,32 @@ conv_halo_kernel(const __grid_constant__ HaloParams p, const __grid_constant__ C
       const uint32_t idesc = tc::Mma<T>::idesc(128, p.N_tile);
       const uint64_t db_w = tc::make_sdesc(smem_w, RB);
       const int w_step16 = p.b_stride / 16;
-      tc::mbar_wait(w_bar, 0);
+      tc::mbar_wait(bar.w, 0);
       int s = 0;
       uint32_t ph = 0;
       int j = 0;
       for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x, ++j) {
         const uint32_t set = (uint32_t)j & 1u;
         const uint32_t use = (uint32_t)j >> 1;
-        tc::mbar_wait(tempty_bar + 8u * set, (use & 1u) ^ 1u);
-        tc::mbar_wait(full_bar + 8u * s, ph);
+        tc::mbar_wait(bar.tempty + 8u * set, (use & 1u) ^ 1u);
+        tc::mbar_wait(bar.full + 8u * s, ph);
         tc::fence_after_sync();
-        if (p.trace && blockIdx.x == 0 && j < 64) p.trace[j * 8 + 2] = clock64();
+        trace_stamp(p.trace, j, 2);
         // descriptors advance by plain 64-bit adds on the 16-byte-unit address field (smem < 256 KB: no carry out
         // of the 14-bit field), so the issue loop is ~4 instructions per tcgen05.mma
         const uint64_t da_stage = tc::make_sdesc(smem_a + (uint32_t)s * p.a_stage_bytes, RB);
         for (int m = 0; m < p.nM; ++m) {
           const uint32_t d_tmem = tmem_base + set * (uint32_t)p.set_stride + (uint32_t)(m * p.N_tile);
           const uint64_t da_m = da_stage + (uint64_t)(m * (128 * RB / 16));
-          {
-            const uint64_t da = da_m + (uint64_t)p.tap_off16[0];
-            tc::Mma<T>::template issue<0>(d_tmem, da, db_w, idesc);
-#pragma unroll
-            for (int k = 1; k < NMMA; ++k) tc::Mma<T>::template issue<1>(d_tmem, da + 2 * k, db_w + 2 * k, idesc);
-          }
+          tc::mma_kchunk<T, NMMA>(d_tmem, da_m + (uint64_t)p.tap_off16[0], db_w, idesc, true);
 #pragma unroll 3
-          for (int tp = 1; tp < p.n_taps; ++tp) {
-            const uint64_t da = da_m + (uint64_t)p.tap_off16[tp];
-            const uint64_t db = db_w + (uint64_t)(tp * w_step16);
-#pragma unroll
-            for (int k = 0; k < NMMA; ++k) tc::Mma<T>::template issue<1>(d_tmem, da + 2 * k, db + 2 * k, idesc);
-          }
+          for (int tp = 1; tp < p.n_taps; ++tp)
+            tc::mma_kchunk<T, NMMA>(d_tmem, da_m + (uint64_t)p.tap_off16[tp], db_w + (uint64_t)(tp * w_step16), idesc,
+                                    false);
         }
-        tc::mma_commit(empty_bar + 8u * s);
-        tc::mma_commit(tfull_bar + 8u * set);
-        if (p.trace && blockIdx.x == 0 && j < 64) p.trace[j * 8 + 3] = clock64();
+        tc::mma_commit(bar.empty + 8u * s);
+        tc::mma_commit(bar.tfull + 8u * set);
+        trace_stamp(p.trace, j, 3);
         if (++s == p.stages) { s = 0; ph ^= 1u; }
       }
     }
@@ -468,7 +454,6 @@ conv_halo_kernel(const __grid_constant__ HaloParams p, const __grid_constant__ C
     const int q = warp & 3;
     const int grp = ((warp - 2) >> 2) & 1;   // accumulator set (tile parity)
     const int half = (warp - 2) >> 3;        // even / odd M tiles of the set
-    const bool tracer = p.trace && blockIdx.x == 0 && threadIdx.x == 64;
     int j = 0;
     for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x, ++j) {
       const uint32_t set = (uint32_t)j & 1u;   // accumulator set == epilogue group
@@ -476,10 +461,10 @@ conv_halo_kernel(const __grid_constant__ HaloParams p, const __grid_constant__ C
       if ((int)set != grp) continue;
       int b, ra, rb, rc, td, th, tw;
       decode(tile, b, ra, rb, rc, td, th, tw);
-      if (tracer && j < 64) p.trace[j * 8 + 4] = clock64();
-      tc::mbar_wait(tfull_bar + 8u * set, use & 1u);
+      trace_stamp(p.trace, j, 4);
+      tc::mbar_wait(bar.tfull + 8u * set, use & 1u);
       tc::fence_after_sync();
-      if (tracer && j < 64) p.trace[j * 8 + 5] = clock64();
+      trace_stamp(p.trace, j, 5);
       for (int m = half; m < p.nM; m += 2) {   // one epilogue group per M tile parity
         const int R = p.R0 + m * 128 + q * 32 + lane;
         const int pw = R % p.PW;
@@ -492,15 +477,7 @@ conv_halo_kernel(const __grid_constant__ HaloParams p, const __grid_constant__ C
         const uint32_t taddr = tmem_base + set * (uint32_t)p.set_stride + (uint32_t)(m * p.N_tile) +
                                ((uint32_t)(q * 32) << 16);
         if (epi_fast_ok(p.epi)) {
-          const EpiRow<T> er = epi_row<T>(p.epi, valid, b, od, oh, ow, 0);
-          uint32_t ra[16];
-          EpiPre pre;
-          for (int c0 = 0; c0 < p.N_tile; c0 += 16) {
-            tc::tmem_ld16_issue(taddr + (uint32_t)c0, ra);
-            epi_prefetch<T>(er, c0, pre);
-            tc::tmem_ld_wait16(ra);
-            epi_finish<T>(er, c0, ra, pre);
-          }
+          epi_drain_fast<T>(epi_row<T>(p.epi, valid, b, od, oh, ow, 0), taddr, 0, p.N_tile);
         } else {
           for (int c0 = 0; c0 < p.N_tile; c0 += 16) {
             float v[16];
@@ -510,16 +487,11 @@ conv_halo_kernel(const __grid_constant__ HaloParams p, const __grid_constant__ C
         }
       }
       tc::fence_before_sync();
-      tc::mbar_arrive(tempty_bar + 8u * set);
-      if (tracer && j < 64) p.trace[j * 8 + 6] = clock64();
+      tc::mbar_arrive(bar.tempty + 8u * set);
+      trace_stamp(p.trace, j, 6);
     }
   }
-  tc::fence_before_sync();
-  __syncthreads();
-  if (warp == 1) {
-    __syncwarp();
-    tc::tmem_dealloc(tmem_base, (uint32_t)p.tmem_cols);
-  }
+  cta_teardown(tmem_base, p.tmem_cols);
 }
 
 
@@ -572,7 +544,6 @@ struct HaloxParams {
   int tmem_cols, set_stride;
   int b_stride, w_bytes;
   int grp_off[9];             // (a*PH + b)*PW: smem row offset of a group's A operand relative to the M tile
-  int pdl;
   long long* trace;
   // plane-ring mode (ring == 1; chosen when the halo box leaves room for ONE stage only, i.e. the TF32 head whose
   // resident weights take 110 KB): the output planes of all columns (image, residue class, H tile) form one sequence
@@ -594,12 +565,7 @@ conv_halox_kernel(const __grid_constant__ HaloxParams p, const __grid_constant__
   const uint32_t smem_w = smem_base;                                   // [n_groups][b_stride] resident weights
   const uint32_t smem_a = smem_w + (uint32_t)p.w_bytes;                 // [stages][a_stage_bytes]
   const uint32_t bar_base = smem_a + (uint32_t)p.stages * p.a_stage_bytes;
-  const uint32_t full_bar = bar_base;            // [4]
-  const uint32_t empty_bar = bar_base + 32u;     // [4]
-  const uint32_t tfull_bar = bar_base + 64u;     // [2]
-  const uint32_t tempty_bar = bar_base + 80u;    // [2]
-  const uint32_t w_bar = bar_base + 96u;
-  const uint32_t tmem_slot = bar_base + 104u;
+  const CtaBarriers bar = cta_barriers(bar_base, kHaloMaxStages);      // ring mode: descriptor table at bar_base + 128
 
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
@@ -610,33 +576,7 @@ conv_halox_kernel(const __grid_constant__ HaloxParams p, const __grid_constant__
   const long long ring_lo = p.ring ? ring_total * blockIdx.x / gridDim.x : 0;
   const long long ring_hi = p.ring ? ring_total * (blockIdx.x + 1) / gridDim.x : 0;
 
-  if (warp == 0 && lane == 0) {
-    tc::prefetch_tmap(&tmA);
-    tc::prefetch_tmap(&tmW);
-    for (int s = 0; s < p.stages; ++s) {
-      tc::mbar_init(full_bar + 8u * s, 1);
-      tc::mbar_init(empty_bar + 8u * s, 1);
-    }
-    for (int a = 0; a < 2; ++a) {
-      tc::mbar_init(tfull_bar + 8u * a, 1);
-      tc::mbar_init(tempty_bar + 8u * a, 256);
-    }
-    tc::mbar_init(w_bar, 1);
-    tc::fence_barrier_init();
-  }
-  if (warp == 1) {
-    __syncwarp();
-    tc::tmem_alloc(tmem_slot, (uint32_t)p.tmem_cols);
-  }
-  tc::fence_before_sync();
-  __syncthreads();
-  tc::fence_after_sync();
-  uint32_t tmem_base;
-  asm volatile("ld.shared.b32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot));
-  if (p.pdl) {
-    asm volatile("griddepcontrol.wait;" ::: "memory");
-    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-  }
+  const uint32_t tmem_base = cta_prologue(bar, p.stages, true, p.tmem_cols, &tmA, &tmW);
 
   // tile -> (batch, (D, H) residue class, sub-grid tile origin)
   auto decode = [&](int tile, int& b, int& ra, int& rb, int& td, int& th) {
@@ -664,9 +604,9 @@ conv_halox_kernel(const __grid_constant__ HaloxParams p, const __grid_constant__
   if (warp == 0) {
     if (lane == 0 && p.ring) {
       // ===== TMA producer, ring mode: weights once, then planes z0-1 .. z1 of every unit, one ring slot each =====
-      tc::mbar_expect_tx(w_bar, (uint32_t)(p.n_groups * p.N_tile * RB));
+      tc::mbar_expect_tx(bar.w, (uint32_t)(p.n_groups * p.N_tile * RB));
       for (int g = 0; g < p.n_groups; ++g)
-        tc::tma_load_2d(smem_w + (uint32_t)g * p.b_stride, &tmW, w_bar, 0, g * p.N_tile);
+        tc::tma_load_2d(smem_w + (uint32_t)g * p.b_stride, &tmW, bar.w, 0, g * p.N_tile);
       uint32_t n = 0;
       for (long long pos = ring_lo; pos < ring_hi;) {
         int b, ra, rb, th, z0, z1;
@@ -674,27 +614,27 @@ conv_halox_kernel(const __grid_constant__ HaloxParams p, const __grid_constant__
         pos += z1 - z0;
         for (int z = z0 - 1; z <= z1; ++z, ++n) {
           const uint32_t slot = n & 3u;
-          if (p.trace && blockIdx.x == 0 && n < 64) p.trace[n * 8 + 0] = clock64();
-          tc::mbar_wait(empty_bar + 8u * slot, ((n >> 2) & 1u) ^ 1u);
-          if (p.trace && blockIdx.x == 0 && n < 64) p.trace[n * 8 + 1] = clock64();
-          tc::mbar_expect_tx(full_bar + 8u * slot, (uint32_t)p.box_bytes);
-          tc::tma_load_5d(smem_a + slot * (uint32_t)p.a_stage_bytes, &tmA, full_bar + 8u * slot, 0, 0,
+          trace_stamp(p.trace, n, 0);
+          tc::mbar_wait(bar.empty + 8u * slot, ((n >> 2) & 1u) ^ 1u);
+          trace_stamp(p.trace, n, 1);
+          tc::mbar_expect_tx(bar.full + 8u * slot, (uint32_t)p.box_bytes);
+          tc::tma_load_5d(smem_a + slot * (uint32_t)p.a_stage_bytes, &tmA, bar.full + 8u * slot, 0, 0,
                           (th * p.BH - p.hh) * d + rb, z * d + ra + p.src_d0, b);
         }
       }
     } else if (lane == 0) {
       // ===== TMA producer: resident weights once, then one halo box per tile =====
-      tc::mbar_expect_tx(w_bar, (uint32_t)(p.n_groups * p.N_tile * RB));
+      tc::mbar_expect_tx(bar.w, (uint32_t)(p.n_groups * p.N_tile * RB));
       for (int g = 0; g < p.n_groups; ++g)
-        tc::tma_load_2d(smem_w + (uint32_t)g * p.b_stride, &tmW, w_bar, 0, g * p.N_tile);
+        tc::tma_load_2d(smem_w + (uint32_t)g * p.b_stride, &tmW, bar.w, 0, g * p.N_tile);
       int s = 0;
       uint32_t ph = 0;
       for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
         int b, ra, rb, td, th;
         decode(tile, b, ra, rb, td, th);
-        tc::mbar_wait(empty_bar + 8u * s, ph ^ 1u);
-        tc::mbar_expect_tx(full_bar + 8u * s, (uint32_t)p.box_bytes);
-        tc::tma_load_5d(smem_a + (uint32_t)s * p.a_stage_bytes, &tmA, full_bar + 8u * s, 0, 0,
+        tc::mbar_wait(bar.empty + 8u * s, ph ^ 1u);
+        tc::mbar_expect_tx(bar.full + 8u * s, (uint32_t)p.box_bytes);
+        tc::tma_load_5d(smem_a + (uint32_t)s * p.a_stage_bytes, &tmA, bar.full + 8u * s, 0, 0,
                         (th * p.BH - p.hh) * d + rb, (td * p.BD - p.hd) * d + ra + p.src_d0, b);
         if (++s == p.stages) { s = 0; ph ^= 1u; }
       }
@@ -714,7 +654,7 @@ conv_halox_kernel(const __grid_constant__ HaloxParams p, const __grid_constant__
           dtab[r * 9 + g] = tc::make_sdesc(smem_a + slot * (uint32_t)p.a_stage_bytes, RB) +
                             (uint64_t)((g < p.n_groups ? p.grp_row[g] : 0) * (RB / 16));
         }
-      tc::mbar_wait(w_bar, 0);
+      tc::mbar_wait(bar.w, 0);
       uint32_t n0 = 0;     // ring index of this unit's first plane (z0 - 1)
       uint32_t j = 0;      // output planes so far == accumulator uses
       for (long long pos = ring_lo; pos < ring_hi;) {
@@ -724,35 +664,27 @@ conv_halox_kernel(const __grid_constant__ HaloxParams p, const __grid_constant__
         const int K = z1 - z0;
         for (int k = 0; k < K; ++k, ++j) {
           const uint32_t set = j & 1u;
-          tc::mbar_wait(tempty_bar + 8u * set, ((j >> 1) & 1u) ^ 1u);
+          tc::mbar_wait(bar.tempty + 8u * set, ((j >> 1) & 1u) ^ 1u);
           for (uint32_t i = (k == 0 ? 0u : 2u); i < 3u; ++i) {     // planes z-1 and z were waited for by plane z-1
             const uint32_t n = n0 + (uint32_t)k + i;
-            tc::mbar_wait(full_bar + 8u * (n & 3u), (n >> 2) & 1u);
+            tc::mbar_wait(bar.full + 8u * (n & 3u), (n >> 2) & 1u);
           }
           tc::fence_after_sync();
-          if (p.trace && blockIdx.x == 0 && j < 64) p.trace[j * 8 + 2] = clock64();
+          trace_stamp(p.trace, j, 2);
           const uint32_t d_tmem = tmem_base + set * (uint32_t)p.set_stride;
           const uint64_t* drow = dtab + ((n0 + (uint32_t)k + 1u) & 3u) * 9u;
           uint64_t dg[9];
 #pragma unroll
           for (int g = 0; g < 9; ++g) dg[g] = drow[g];
 #pragma unroll
-          for (int g = 0; g < 9; ++g) {
-            if (g < p.n_groups) {
-              const uint64_t da = dg[g];
-              const uint64_t db = db_w + (uint64_t)(g * w_step16);
-              if (g == 0) tc::Mma<T>::template issue<0>(d_tmem, da, db, idesc);
-              else tc::Mma<T>::template issue<1>(d_tmem, da, db, idesc);
-#pragma unroll
-              for (int kk = 1; kk < NMMA; ++kk) tc::Mma<T>::template issue<1>(d_tmem, da + 2 * kk, db + 2 * kk, idesc);
-            }
-          }
-          tc::mma_commit(tfull_bar + 8u * set);
-          if (p.trace && blockIdx.x == 0 && j < 64) p.trace[j * 8 + 3] = clock64();
-          tc::mma_commit(empty_bar + 8u * ((n0 + (uint32_t)k) & 3u));            // plane z-1 is done with
+          for (int g = 0; g < 9; ++g)
+            if (g < p.n_groups) tc::mma_kchunk<T, NMMA>(d_tmem, dg[g], db_w + (uint64_t)(g * w_step16), idesc, g == 0);
+          tc::mma_commit(bar.tfull + 8u * set);
+          trace_stamp(p.trace, j, 3);
+          tc::mma_commit(bar.empty + 8u * ((n0 + (uint32_t)k) & 3u));            // plane z-1 is done with
           if (k == K - 1) {                                                       // ... and the unit's last two
-            tc::mma_commit(empty_bar + 8u * ((n0 + (uint32_t)k + 1u) & 3u));
-            tc::mma_commit(empty_bar + 8u * ((n0 + (uint32_t)k + 2u) & 3u));
+            tc::mma_commit(bar.empty + 8u * ((n0 + (uint32_t)k + 1u) & 3u));
+            tc::mma_commit(bar.empty + 8u * ((n0 + (uint32_t)k + 2u) & 3u));
           }
         }
         n0 += (uint32_t)K + 2u;
@@ -762,37 +694,30 @@ conv_halox_kernel(const __grid_constant__ HaloxParams p, const __grid_constant__
       const uint32_t idesc = tc::Mma<T>::idesc(128, p.N_tile);
       const uint64_t db_w = tc::make_sdesc(smem_w, RB);
       const int w_step16 = p.b_stride / 16;
-      tc::mbar_wait(w_bar, 0);
+      tc::mbar_wait(bar.w, 0);
       int s = 0;
       uint32_t ph = 0;
       int j = 0;
       for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x, ++j) {
         const uint32_t set = (uint32_t)j & 1u;
         const uint32_t use = (uint32_t)j >> 1;
-        tc::mbar_wait(tempty_bar + 8u * set, (use & 1u) ^ 1u);
-        tc::mbar_wait(full_bar + 8u * s, ph);
+        tc::mbar_wait(bar.tempty + 8u * set, (use & 1u) ^ 1u);
+        tc::mbar_wait(bar.full + 8u * s, ph);
         tc::fence_after_sync();
-        if (p.trace && blockIdx.x == 0 && j < 64) p.trace[j * 8 + 2] = clock64();
+        trace_stamp(p.trace, j, 2);
         const uint64_t da_stage = tc::make_sdesc(smem_a + (uint32_t)s * p.a_stage_bytes, RB);
         for (int m = 0; m < p.nM; ++m) {
           const uint32_t d_tmem = tmem_base + set * (uint32_t)p.set_stride + (uint32_t)(m * p.N_tile);
-          {
-            const uint64_t da = da_stage + (uint64_t)((p.mt_row[m] + p.grp_off[0]) * (RB / 16));
-            tc::Mma<T>::template issue<0>(d_tmem, da, db_w, idesc);
-#pragma unroll
-            for (int k = 1; k < NMMA; ++k) tc::Mma<T>::template issue<1>(d_tmem, da + 2 * k, db_w + 2 * k, idesc);
-          }
+          tc::mma_kchunk<T, NMMA>(d_tmem, da_stage + (uint64_t)((p.mt_row[m] + p.grp_off[0]) * (RB / 16)), db_w, idesc,
+                                  true);
 #pragma unroll 2
-          for (int g = 1; g < p.n_groups; ++g) {
-            const uint64_t da = da_stage + (uint64_t)((p.mt_row[m] + p.grp_off[g]) * (RB / 16));
-            const uint64_t db = db_w + (uint64_t)(g * w_step16);
-#pragma unroll
-            for (int k = 0; k < NMMA; ++k) tc::Mma<T>::template issue<1>(d_tmem, da + 2 * k, db + 2 * k, idesc);
-          }
+          for (int g = 1; g < p.n_groups; ++g)
+            tc::mma_kchunk<T, NMMA>(d_tmem, da_stage + (uint64_t)((p.mt_row[m] + p.grp_off[g]) * (RB / 16)),
+                                    db_w + (uint64_t)(g * w_step16), idesc, false);
         }
-        tc::mma_commit(empty_bar + 8u * s);
-        tc::mma_commit(tfull_bar + 8u * set);
-        if (p.trace && blockIdx.x == 0 && j < 64) p.trace[j * 8 + 3] = clock64();
+        tc::mma_commit(bar.empty + 8u * s);
+        tc::mma_commit(bar.tfull + 8u * set);
+        trace_stamp(p.trace, j, 3);
         if (++s == p.stages) { s = 0; ph ^= 1u; }
       }
     }
@@ -809,7 +734,6 @@ conv_halox_kernel(const __grid_constant__ HaloxParams p, const __grid_constant__
     const bool lo_ok = pw >= d, hi_ok = pw + d < p.PW;
     const int chunks = p.CP >> 4;
     const int n_items = p.nM * chunks;
-    const bool tracer = p.trace && blockIdx.x == 0 && threadIdx.x == 64;
     if (p.ring) {
       // ring mode: one M tile (one plane, 128 / PW h-rows) per accumulator use
       uint32_t jr = 0;
@@ -820,10 +744,10 @@ conv_halox_kernel(const __grid_constant__ HaloxParams p, const __grid_constant__
         for (int z = z0; z < z1; ++z, ++jr) {
           const uint32_t set = jr & 1u;
           if ((int)set != grp) continue;
-          if (tracer && jr < 64) p.trace[jr * 8 + 4] = clock64();
-          tc::mbar_wait(tfull_bar + 8u * set, (jr >> 1) & 1u);
+          trace_stamp(p.trace, jr, 4);
+          tc::mbar_wait(bar.tfull + 8u * set, (jr >> 1) & 1u);
           tc::fence_after_sync();
-          if (tracer && jr < 64) p.trace[jr * 8 + 5] = clock64();
+          trace_stamp(p.trace, jr, 5);
           const int od = z * d + ra;
           const int oh = (th * p.BH + hr) * d + rb;
           const bool valid = od < p.D && oh < p.H;
@@ -835,8 +759,8 @@ conv_halox_kernel(const __grid_constant__ HaloxParams p, const __grid_constant__
             if (valid) conv_epilogue_row<T, 16>(p.epi, b, od, oh, pw, c0, v);
           }
           tc::fence_before_sync();
-          tc::mbar_arrive(tempty_bar + 8u * set);
-          if (tracer && jr < 64) p.trace[jr * 8 + 6] = clock64();
+          tc::mbar_arrive(bar.tempty + 8u * set);
+          trace_stamp(p.trace, jr, 6);
         }
       }
     }
@@ -847,10 +771,10 @@ conv_halox_kernel(const __grid_constant__ HaloxParams p, const __grid_constant__
       if ((int)set != grp) continue;
       int b, ra, rb, td, th;
       decode(tile, b, ra, rb, td, th);
-      if (tracer && j < 64) p.trace[j * 8 + 4] = clock64();
-      tc::mbar_wait(tfull_bar + 8u * set, use & 1u);
+      trace_stamp(p.trace, j, 4);
+      tc::mbar_wait(bar.tfull + 8u * set, use & 1u);
       tc::fence_after_sync();
-      if (tracer && j < 64) p.trace[j * 8 + 5] = clock64();
+      trace_stamp(p.trace, j, 5);
       for (int it = half; it < n_items; it += 2) {
         const int m = it / chunks, c0 = (it - m * chunks) * 16;
         const int od = (td * p.BD + p.mt_pd[m] - p.hd) * d + ra;
@@ -863,16 +787,11 @@ conv_halox_kernel(const __grid_constant__ HaloxParams p, const __grid_constant__
         if (valid) conv_epilogue_row<T, 16>(p.epi, b, od, oh, pw, c0, v);
       }
       tc::fence_before_sync();
-      tc::mbar_arrive(tempty_bar + 8u * set);
-      if (tracer && j < 64) p.trace[j * 8 + 6] = clock64();
+      tc::mbar_arrive(bar.tempty + 8u * set);
+      trace_stamp(p.trace, j, 6);
     }
   }
-  tc::fence_before_sync();
-  __syncthreads();
-  if (warp == 1) {
-    __syncwarp();
-    tc::tmem_dealloc(tmem_base, (uint32_t)p.tmem_cols);
-  }
+  cta_teardown(tmem_base, p.tmem_cols);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1008,29 +927,7 @@ static int fill_epi(const occd_conv_desc* d, ConvEpi* e) {
   e->res2_cstride = d->res2_cstride; e->res2_coff = d->res2_coff; e->res2_post = d->res2_post;
   e->out1_mode = d->out1_mode; e->out1 = d->out1;
   e->out1_cstride = d->out1_cstride; e->out1_coff = d->out1_coff; e->out1_C = d->out1_C;
-  { const char* v = getenv("OCCD_DEBUG_EPI"); e->dbg = v ? atoi(v) : 0; }
   return 0;
-}
-
-// Programmatic dependent launch (common.cuh): the conv kernels wait on griddepcontrol after their prologue (barrier
-// init, TMEM alloc, tensor-map prefetch overlap the tail of the previous grid).  Measured on B200 (round 2,
-// profiles/r02_ab_experiments.txt): 1.0 % of the config-2 forward, results bit-identical.
-static int pdl_enabled() { return occd_pdl_enabled(); }
-
-template <typename... KArgs, typename... Args>
-static cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, int threads, size_t smem, cudaStream_t st,
-                              Args&&... args) {
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = grid;
-  cfg.blockDim = dim3((unsigned)threads);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  return cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
 }
 
 static int n_sms_current() {
@@ -1045,26 +942,109 @@ static int n_sms_current() {
   return n_sms[dev];
 }
 
-// Halo-tile plan: stride-1 "same" convolution whose taps are {-d,0,d} offsets, one source, one k-chunk, one N tile.
-// halo_geometry is pure host arithmetic; halo_encode builds the tensor maps.
-static int halo_geometry(const occd_conv_desc* d, occd_conv_plan* pl) {
-#define HALO_REQUIRE(cond, msg) do { if (!(cond)) { occd_set_last_error("occd_conv_plan_create(halo): " msg); return OCCD_ERR_UNSUPPORTED; } } while (0)
-  HALO_REQUIRE(d->n_src == 1, "one source only");
-  HALO_REQUIRE(d->stride[0] == 1 && d->stride[1] == 1 && d->stride[2] == 1, "stride must be 1");
-  HALO_REQUIRE(d->omul[0] == 1 && d->omul[1] == 1 && d->omul[2] == 1 && d->oadd[0] == 0 && d->oadd[1] == 0 &&
-               d->oadd[2] == 0, "identity output mapping only");
-  HALO_REQUIRE(d->OD + 2 * d->src_d0 == d->ID && d->OH == d->IH && d->OW == d->IW,
+// persistent kernels: one CTA per SM, fewer when there are fewer tiles
+static int persistent_grid(occd_conv_plan* pl, long long num_tiles) {
+  if (num_tiles >= 2147483647LL) {
+    occd_set_last_error("occd_conv_plan_create: too many tiles");
+    return OCCD_ERR_UNSUPPORTED;
+  }
+  const int n_sms = n_sms_current();
+  pl->grid = dim3((unsigned)(num_tiles < n_sms ? num_tiles : n_sms));
+  return OCCD_OK;
+}
+
+static CUtensorMapSwizzle swizzle_for(int rb) {
+  return rb == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : (rb == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B);
+}
+
+static CUtensorMapDataType tm_dtype(int dtype) {
+  return dtype == OCCD_DTYPE_F32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+}
+
+// Tensor maps of a tcgen05 plan.  Source s: 5-D (channels, W, H, D, B) over its channel window; a box is one K chunk of
+// channels x box[] positions, visited with traversal strides estr[] (box and estr in W, H, D order).  Weights: 2-D
+// (Kpad, rows); a box is one K chunk x w_box_rows rows.
+static int encode_maps(const occd_conv_desc* d, occd_conv_plan* pl, const int box[3], const int estr[3],
+                       int w_box_rows) {
+  EncodeTiledFn enc = get_encode_fn();
+  if (!enc) {
+    occd_set_last_error("occd_conv_plan_create: cuTensorMapEncodeTiled unavailable (no CUDA driver / GPU?)");
+    return OCCD_ERR_CUDA;
+  }
+  const int es = pl->esize;
+  const CUtensorMapSwizzle sw = swizzle_for(pl->rb);
+  char msg[160];
+  for (int s = 0; s < d->n_src; ++s) {
+    const cuuint64_t cs = (cuuint64_t)d->src_cstride[s] * es;
+    cuuint64_t gdim[5] = {(cuuint64_t)d->src_C[s], (cuuint64_t)d->IW, (cuuint64_t)d->IH, (cuuint64_t)d->ID,
+                          (cuuint64_t)d->B};
+    cuuint64_t gstr[4] = {cs, cs * d->IW, cs * d->IW * d->IH, cs * d->IW * d->IH * d->ID};
+    cuuint32_t bx[5] = {(cuuint32_t)pl->kc, (cuuint32_t)box[0], (cuuint32_t)box[1], (cuuint32_t)box[2], 1};
+    cuuint32_t ex[5] = {1, (cuuint32_t)estr[0], (cuuint32_t)estr[1], (cuuint32_t)estr[2], 1};
+    void* base = (void*)((const char*)d->src[s] + (size_t)d->src_coff[s] * es);
+    CUresult r = enc(&pl->tmA[s], tm_dtype(pl->dtype), 5, base, gdim, gstr, bx, ex, CU_TENSOR_MAP_INTERLEAVE_NONE, sw,
+                     CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    if (r != CUDA_SUCCESS) {
+      snprintf(msg, sizeof(msg), "occd_conv_plan_create: cuTensorMapEncodeTiled(source %d) failed with %d", s, (int)r);
+      occd_set_last_error(msg);
+      return OCCD_ERR_CUDA;
+    }
+  }
+  for (int s = d->n_src; s < OCCD_CONV_MAX_SRC; ++s) pl->tmA[s] = pl->tmA[0];
+  cuuint64_t gdim[2] = {(cuuint64_t)d->Kpad, (cuuint64_t)d->n_taps * d->Cout_pad * (d->weight_per_image ? d->B : 1)};
+  cuuint64_t gstr[1] = {(cuuint64_t)d->Kpad * es};
+  cuuint32_t bx[2] = {(cuuint32_t)pl->kc, (cuuint32_t)w_box_rows};
+  cuuint32_t ex[2] = {1, 1};
+  CUresult r = enc(&pl->tmW, tm_dtype(pl->dtype), 2, (void*)d->weight, gdim, gstr, bx, ex,
+                   CU_TENSOR_MAP_INTERLEAVE_NONE, sw, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS) {
+    snprintf(msg, sizeof(msg), "occd_conv_plan_create: cuTensorMapEncodeTiled(weights) failed with %d", (int)r);
+    occd_set_last_error(msg);
+    return OCCD_ERR_CUDA;
+  }
+  return OCCD_OK;
+}
+
+// refusal of an impl whose kernel cannot run the described conv ("occd_conv_plan_create(<tag>): <msg>")
+static int refuse(const char* tag, const char* msg) {
+  char buf[256];
+  snprintf(buf, sizeof(buf), "occd_conv_plan_create(%s): %s", tag, msg);
+  occd_set_last_error(buf);
+  return OCCD_ERR_UNSUPPORTED;
+}
+#define PLAN_REQUIRE(cond, tag, msg) do { if (!(cond)) return refuse(tag, msg); } while (0)
+
+// preconditions shared by the halo kernels: a stride-1 "same" convolution of one source whose channels are one K chunk
+// (Kpad == the chunk); sets the plan's K chunk
+static int same_grid_one_chunk(const occd_conv_desc* d, occd_conv_plan* pl, const char* tag) {
+  PLAN_REQUIRE(d->n_src == 1, tag, "one source only");
+  PLAN_REQUIRE(d->stride[0] == 1 && d->stride[1] == 1 && d->stride[2] == 1, tag, "stride must be 1");
+  PLAN_REQUIRE(d->omul[0] == 1 && d->omul[1] == 1 && d->omul[2] == 1 && d->oadd[0] == 0 && d->oadd[1] == 0 &&
+               d->oadd[2] == 0, tag, "identity output mapping only");
+  PLAN_REQUIRE(d->OD + 2 * d->src_d0 == d->ID && d->OH == d->IH && d->OW == d->IW, tag,
                "output grid must equal the input grid (plus symmetric halo margins)");
-  HALO_REQUIRE(d->n_taps <= 27, "at most 27 taps");
-  HALO_REQUIRE(d->src_C[0] <= 128 / pl->esize && d->Cout_pad <= 128,
-               "channel counts too large for the resident-weight scheme (one K chunk)");
+  const int KC = chunk_channels(d->src_C[0], pl->esize);
+  PLAN_REQUIRE(d->src_C[0] <= KC && d->Kpad == KC, tag, "one K chunk: Kpad must equal the k-chunk");
+  pl->kc = KC;
+  pl->rb = KC * pl->esize;
+  return OCCD_OK;
+}
+
+// Halo-tile plan (conv_halo_kernel): stride-1 "same" convolution whose taps are {-d,0,d} offsets, one source, one
+// k-chunk, one N tile.  Host arithmetic, then the tensor maps.
+static int plan_halo(const occd_conv_desc* d, occd_conv_plan* pl) {
+  const int rc = same_grid_one_chunk(d, pl, "halo");
+  if (rc != OCCD_OK) return rc;
+  PLAN_REQUIRE(d->n_taps <= 27, "halo", "at most 27 taps");
+  PLAN_REQUIRE(d->Cout_pad <= 128, "halo", "Cout_pad too large for the resident-weight scheme");
   int dil = 0;
   for (int i = 0; i < d->n_taps; ++i) {
     const int o[3] = {abs(d->taps[i].dz), abs(d->taps[i].dy), abs(d->taps[i].dx)};
     for (int k = 0; k < 3; ++k)
-      if (o[k]) { if (!dil) dil = o[k]; HALO_REQUIRE(o[k] == dil, "taps must be {-d,0,d} offsets"); }
+      if (o[k]) { if (!dil) dil = o[k]; PLAN_REQUIRE(o[k] == dil, "halo", "taps must be {-d,0,d} offsets"); }
   }
-  HALO_REQUIRE(dil >= 1 && dil <= 8, "dilation must be 1..8");
+  PLAN_REQUIRE(dil >= 1 && dil <= 8, "halo", "dilation must be 1..8");
   int hal[3] = {0, 0, 0};
   for (int i = 0; i < d->n_taps; ++i) {
     if (d->taps[i].dz) hal[0] = 1;
@@ -1073,10 +1053,6 @@ static int halo_geometry(const occd_conv_desc* d, occd_conv_plan* pl) {
   }
   HaloParams& h = pl->halo;
   fill_epi(d, &h.epi);
-  const int KC = chunk_channels(d->src_C[0], pl->esize);
-  HALO_REQUIRE(d->Kpad == KC, "Kpad must equal the k-chunk");
-  pl->kc = KC;
-  pl->rb = KC * pl->esize;
   const int row_bytes = pl->rb;
   h.d = dil; h.D = d->OD; h.H = d->IH; h.W = d->IW;
   h.src_d0 = d->src_d0;
@@ -1085,7 +1061,7 @@ static int halo_geometry(const occd_conv_desc* d, occd_conv_plan* pl) {
   h.N_tile = d->Cout_pad;
   h.b_stride = round_up(h.N_tile * row_bytes, 1024);
   h.w_bytes = h.n_taps * h.b_stride;
-  HALO_REQUIRE(h.w_bytes <= 112 * 1024, "weights do not fit in shared memory");
+  PLAN_REQUIRE(h.w_bytes <= 112 * 1024, "halo", "weights do not fit in shared memory");
   const int sD = (d->OD + dil - 1) / dil, sH = (d->IH + dil - 1) / dil, sW = (d->IW + dil - 1) / dil;
   const int smem_total = 224 * 1024 - h.w_bytes - 2048;
   // W extent of the box: the whole sub-sampled line when it fits, else equal splits of at most 62
@@ -1113,7 +1089,7 @@ static int halo_geometry(const occd_conv_desc* d, occd_conv_plan* pl) {
         h.R0 = R0; h.nM = nM; h.a_stage_bytes = stage;
       }
     }
-  HALO_REQUIRE(best_cost >= 0, "no tile shape fits");
+  PLAN_REQUIRE(best_cost >= 0, "halo", "no tile shape fits");
   h.tilesD = (sD + h.BD - 1) / h.BD; h.tilesH = (sH + h.BH - 1) / h.BH; h.tilesW = nW;
   h.box_bytes = h.PD * h.PH * h.PW * row_bytes;
   h.stages = smem_total / h.a_stage_bytes;
@@ -1125,46 +1101,37 @@ static int halo_geometry(const occd_conv_desc* d, occd_conv_plan* pl) {
     h.tap_off16[i] = (h.R0 + ((d->taps[i].dz / dil) * h.PH + d->taps[i].dy / dil) * h.PW + d->taps[i].dx / dil) *
                      row_bytes / 16;
   h.trace = g_trace_buf;
-  h.pdl = pdl_enabled();
   pl->smem = (size_t)h.w_bytes + (size_t)h.stages * h.a_stage_bytes + 128 + 1024;
-  const long long num_tiles = (long long)d->B * dil * dil * dil * h.tilesD * h.tilesH * h.tilesW;
-  HALO_REQUIRE(num_tiles < 2147483647LL, "too many tiles");
-  const int n_sms = n_sms_current();
-  pl->grid = dim3((unsigned)(num_tiles < n_sms ? num_tiles : n_sms));
-#undef HALO_REQUIRE
-  return OCCD_OK;
+  const int rg = persistent_grid(pl, (long long)d->B * dil * dil * dil * h.tilesD * h.tilesH * h.tilesW);
+  if (rg != OCCD_OK) return rg;
+  const int box[3] = {(h.PW - 1) * dil + 1, (h.PH - 1) * dil + 1, (h.PD - 1) * dil + 1};
+  const int estr[3] = {dil, dil, dil};
+  return encode_maps(d, pl, box, estr, h.N_tile);
 }
 
 
-// x-packed halo plan (conv_halox_kernel): host arithmetic
-static int halox_geometry(const occd_conv_desc* d, occd_conv_plan* pl) {
-#define HX_REQUIRE(cond, msg) do { if (!(cond)) { occd_set_last_error("occd_conv_plan_create(halox): " msg); return OCCD_ERR_UNSUPPORTED; } } while (0)
-  HX_REQUIRE(d->n_src == 1 && !d->weight_per_image, "one source, shared weights");
-  HX_REQUIRE(d->stride[0] == 1 && d->stride[1] == 1 && d->stride[2] == 1, "stride must be 1");
-  HX_REQUIRE(d->omul[0] == 1 && d->omul[1] == 1 && d->omul[2] == 1 && d->oadd[0] == 0 && d->oadd[1] == 0 &&
-             d->oadd[2] == 0, "identity output mapping only");
-  HX_REQUIRE(d->OD + 2 * d->src_d0 == d->ID && d->OH == d->IH && d->OW == d->IW,
-             "output grid must equal the input grid (plus symmetric halo margins)");
-  HX_REQUIRE(d->IW == 8 || d->IW == 16 || d->IW == 32, "innermost extent W must be 8, 16 or 32 (one warp row)");
-  HX_REQUIRE(d->n_taps % 3 == 0 && d->n_taps <= 27, "taps must come as W triples");
-  HX_REQUIRE(d->src_C[0] <= 128 / pl->esize && 3 * d->Cout_pad <= 256, "one K chunk, 3 * Cout_pad <= 256");
+// x-packed halo plan (conv_halox_kernel): host arithmetic, then the tensor maps
+static int plan_halox(const occd_conv_desc* d, occd_conv_plan* pl) {
+  const int rc = same_grid_one_chunk(d, pl, "halox");
+  if (rc != OCCD_OK) return rc;
+  PLAN_REQUIRE(d->IW == 8 || d->IW == 16 || d->IW == 32, "halox",
+               "innermost extent W must be 8, 16 or 32 (one warp row)");
+  PLAN_REQUIRE(d->n_taps % 3 == 0 && d->n_taps <= 27, "halox", "taps must come as W triples");
+  PLAN_REQUIRE(3 * d->Cout_pad <= 256, "halox", "3 * Cout_pad <= 256");
   const int dil = d->taps[2].dx;
-  HX_REQUIRE(dil >= 1 && dil <= 8 && dil < d->IW, "W dilation");
+  PLAN_REQUIRE(dil >= 1 && dil <= 8 && dil < d->IW, "halox", "W dilation");
   int hal[2] = {0, 0};
   for (int i = 0; i < d->n_taps; i += 3) {
     const occd_conv_tap &a = d->taps[i], &b = d->taps[i + 1], &c = d->taps[i + 2];
-    HX_REQUIRE(a.dx == -dil && b.dx == 0 && c.dx == dil && a.dz == b.dz && a.dz == c.dz && a.dy == b.dy &&
-               a.dy == c.dy, "taps must be ordered (dz, dy) groups of dx = -d, 0, +d");
-    HX_REQUIRE((a.dz == 0 || abs(a.dz) == dil) && (a.dy == 0 || abs(a.dy) == dil), "D / H taps must be {-d, 0, d}");
+    PLAN_REQUIRE(a.dx == -dil && b.dx == 0 && c.dx == dil && a.dz == b.dz && a.dz == c.dz && a.dy == b.dy &&
+                 a.dy == c.dy, "halox", "taps must be ordered (dz, dy) groups of dx = -d, 0, +d");
+    PLAN_REQUIRE((a.dz == 0 || abs(a.dz) == dil) && (a.dy == 0 || abs(a.dy) == dil), "halox",
+                 "D / H taps must be {-d, 0, d}");
     if (a.dz) hal[0] = 1;
     if (a.dy) hal[1] = 1;
   }
   HaloxParams& h = pl->halox;
   fill_epi(d, &h.epi);
-  const int KC = chunk_channels(d->src_C[0], pl->esize);
-  HX_REQUIRE(d->Kpad == KC, "Kpad must equal the k-chunk");
-  pl->kc = KC;
-  pl->rb = KC * pl->esize;
   const int RB = pl->rb, NMMA = RB / 32;
   h.d = dil; h.D = d->OD; h.H = d->IH;
   h.src_d0 = d->src_d0;
@@ -1176,7 +1143,7 @@ static int halox_geometry(const occd_conv_desc* d, occd_conv_plan* pl) {
   h.b_stride = round_up(h.N_tile * RB, 1024);
   h.w_bytes = h.n_groups * h.b_stride;
   const int smem_total = 227 * 1024 - h.w_bytes - 4096;   // barriers, TMEM slot, 1024-byte alignment slack
-  HX_REQUIRE(smem_total > 0, "weights do not fit in shared memory");
+  PLAN_REQUIRE(smem_total > 0, "halox", "weights do not fit in shared memory");
   const int HR = 128 / h.PW;                               // h-rows of one plane per M tile
   const int sD = (d->OD + dil - 1) / dil, sH = (d->IH + dil - 1) / dil;
   // CTA tile = BD planes x nB blocks of HR h-rows (<= 2 M tiles: two accumulator sets of nM x N_tile columns)
@@ -1208,15 +1175,13 @@ static int halox_geometry(const occd_conv_desc* d, occd_conv_plan* pl) {
       h.set_stride = set_stride;
     }
   }
-  HX_REQUIRE(best >= 0, "no tile shape fits");
+  PLAN_REQUIRE(best >= 0, "halox", "no tile shape fits");
   h.ring = 0;
   {
-    // plane ring instead of a single-stage box (see HaloxParams): needs D taps and four single-plane stages.
-    // OCCD_HALOX_RING=0 keeps the box (experiment hook, tools/conv_bench.py)
-    static const bool ring_off = [] { const char* e = getenv("OCCD_HALOX_RING"); return e && atoi(e) == 0; }();
+    // plane ring instead of a single-stage box (see HaloxParams): needs D taps and four single-plane stages
     const int PHr = HR + 2 * hal[1];
     const int plane = round_up(PHr * h.PW * RB, 1024);
-    if (!ring_off && h.stages < 2 && hal[0] == 1 && 4 * plane <= smem_total && (PHr - 1) * dil + 1 <= 256) {
+    if (h.stages < 2 && hal[0] == 1 && 4 * plane <= smem_total && (PHr - 1) * dil + 1 <= 256) {
       h.ring = 1;
       h.BD = 1; h.BH = HR; h.PD = 3; h.PH = PHr; h.nM = 1;
       h.a_stage_bytes = plane; h.stages = 4;
@@ -1245,98 +1210,18 @@ static int halox_geometry(const occd_conv_desc* d, occd_conv_plan* pl) {
   h.sD = sD;
   h.n_cols = d->B * dil * dil * h.tilesH;
   h.trace = g_trace_buf;
-  h.pdl = pdl_enabled();
   pl->smem = (size_t)h.w_bytes + (size_t)h.stages * h.a_stage_bytes + 128 + 512 + 1024;   // barriers, ring-mode descriptor table, alignment slack
   const long long num_tiles = h.ring ? (long long)h.n_cols * sD      // ring mode: M tiles; each CTA takes a contiguous share
                                      : (long long)d->B * dil * dil * h.tilesD * h.tilesH;
-  HX_REQUIRE(num_tiles < 2147483647LL, "too many tiles");
-  const int n_sms = n_sms_current();
-  pl->grid = dim3((unsigned)(num_tiles < n_sms ? num_tiles : n_sms));
-#undef HX_REQUIRE
-  return OCCD_OK;
+  const int rg = persistent_grid(pl, num_tiles);
+  if (rg != OCCD_OK) return rg;
+  const int box[3] = {h.PW, (h.PH - 1) * dil + 1, h.ring ? 1 : (h.PD - 1) * dil + 1};   // ring mode: one plane per load
+  const int estr[3] = {1, dil, dil};
+  return encode_maps(d, pl, box, estr, h.N_tile);
 }
 
-static CUtensorMapSwizzle swizzle_for(int rb) {
-  return rb == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : (rb == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B);
-}
-
-static CUtensorMapDataType tm_dtype(int dtype) {
-  return dtype == OCCD_DTYPE_F32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
-}
-
-static int halo_encode(const occd_conv_desc* d, occd_conv_plan* pl) {
-  const HaloParams& h = pl->halo;
-  const int KC = pl->kc, C = d->src_C[0], dil = h.d, es = pl->esize;
-  EncodeTiledFn enc = get_encode_fn();
-  if (!enc) {
-    occd_set_last_error("occd_conv_plan_create: cuTensorMapEncodeTiled unavailable (no CUDA driver / GPU?)");
-    return OCCD_ERR_CUDA;
-  }
-  const CUtensorMapSwizzle sw = swizzle_for(pl->rb);
-  {
-    const cuuint64_t cs = (cuuint64_t)d->src_cstride[0] * es;
-    cuuint64_t gdim[5] = {(cuuint64_t)C, (cuuint64_t)d->IW, (cuuint64_t)d->IH, (cuuint64_t)d->ID, (cuuint64_t)d->B};
-    cuuint64_t gstr[4] = {cs, cs * d->IW, cs * d->IW * d->IH, cs * d->IW * d->IH * d->ID};
-    cuuint32_t box[5] = {(cuuint32_t)KC, (cuuint32_t)((h.PW - 1) * dil + 1), (cuuint32_t)((h.PH - 1) * dil + 1),
-                         (cuuint32_t)((h.PD - 1) * dil + 1), 1};
-    cuuint32_t estr[5] = {1, (cuuint32_t)dil, (cuuint32_t)dil, (cuuint32_t)dil, 1};
-    void* base = (void*)((const char*)d->src[0] + (size_t)d->src_coff[0] * es);
-    CUresult r = enc(&pl->tmA[0], tm_dtype(pl->dtype), 5, base, gdim, gstr, box, estr,
-                     CU_TENSOR_MAP_INTERLEAVE_NONE, sw, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) { occd_set_last_error("occd_conv_plan_create(halo): cuTensorMapEncodeTiled(source) failed"); return OCCD_ERR_CUDA; }
-  }
-  {
-    cuuint64_t gdim[2] = {(cuuint64_t)d->Kpad, (cuuint64_t)d->n_taps * d->Cout_pad};
-    cuuint64_t gstr[1] = {(cuuint64_t)d->Kpad * es};
-    cuuint32_t box[2] = {(cuuint32_t)KC, (cuuint32_t)h.N_tile};
-    cuuint32_t estr[2] = {1, 1};
-    CUresult r = enc(&pl->tmW, tm_dtype(pl->dtype), 2, (void*)d->weight, gdim, gstr, box, estr,
-                     CU_TENSOR_MAP_INTERLEAVE_NONE, sw, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) { occd_set_last_error("occd_conv_plan_create(halo): cuTensorMapEncodeTiled(weights) failed"); return OCCD_ERR_CUDA; }
-  }
-  return OCCD_OK;
-}
-
-
-static int halox_encode(const occd_conv_desc* d, occd_conv_plan* pl) {
-  const HaloxParams& h = pl->halox;
-  const int KC = pl->kc, C = d->src_C[0], dil = h.d, es = pl->esize;
-  EncodeTiledFn enc = get_encode_fn();
-  if (!enc) {
-    occd_set_last_error("occd_conv_plan_create: cuTensorMapEncodeTiled unavailable (no CUDA driver / GPU?)");
-    return OCCD_ERR_CUDA;
-  }
-  const CUtensorMapSwizzle sw = swizzle_for(pl->rb);
-  {
-    const cuuint64_t cs = (cuuint64_t)d->src_cstride[0] * es;
-    cuuint64_t gdim[5] = {(cuuint64_t)C, (cuuint64_t)d->IW, (cuuint64_t)d->IH, (cuuint64_t)d->ID, (cuuint64_t)d->B};
-    cuuint64_t gstr[4] = {cs, cs * d->IW, cs * d->IW * d->IH, cs * d->IW * d->IH * d->ID};
-    cuuint32_t box[5] = {(cuuint32_t)KC, (cuuint32_t)h.PW, (cuuint32_t)((h.PH - 1) * dil + 1),
-                         (cuuint32_t)(h.ring ? 1 : (h.PD - 1) * dil + 1), 1};   // ring mode: one plane per load
-    cuuint32_t estr[5] = {1, 1, (cuuint32_t)dil, (cuuint32_t)dil, 1};
-    void* base = (void*)((const char*)d->src[0] + (size_t)d->src_coff[0] * es);
-    CUresult r = enc(&pl->tmA[0], tm_dtype(pl->dtype), 5, base, gdim, gstr, box, estr,
-                     CU_TENSOR_MAP_INTERLEAVE_NONE, sw, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) { occd_set_last_error("occd_conv_plan_create(halox): cuTensorMapEncodeTiled(source) failed"); return OCCD_ERR_CUDA; }
-  }
-  {
-    cuuint64_t gdim[2] = {(cuuint64_t)d->Kpad, (cuuint64_t)d->n_taps * d->Cout_pad};
-    cuuint64_t gstr[1] = {(cuuint64_t)d->Kpad * es};
-    cuuint32_t box[2] = {(cuuint32_t)KC, (cuuint32_t)h.N_tile};
-    cuuint32_t estr[2] = {1, 1};
-    CUresult r = enc(&pl->tmW, tm_dtype(pl->dtype), 2, (void*)d->weight, gdim, gstr, box, estr,
-                     CU_TENSOR_MAP_INTERLEAVE_NONE, sw, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) { occd_set_last_error("occd_conv_plan_create(halox): cuTensorMapEncodeTiled(weights) failed"); return OCCD_ERR_CUDA; }
-  }
-  return OCCD_OK;
-}
-
-// Per-tap (TC) plan: host arithmetic only; tc_encode builds the tensor maps.  xp: x-packed variant (TCX)
-static int tc_geometry(const occd_conv_desc* d, occd_conv_plan* pl, bool xp) {
+// Per-tap (TC) plan: host arithmetic, then the tensor maps.  xp: x-packed variant (TCX)
+static int plan_tc(const occd_conv_desc* d, occd_conv_plan* pl, bool xp) {
   int maxC = 0;
   for (int s = 0; s < d->n_src; ++s) maxC = d->src_C[s] > maxC ? d->src_C[s] : maxC;
   TcParams& t = pl->tc;
@@ -1441,9 +1326,7 @@ static int tc_geometry(const occd_conv_desc* d, occd_conv_plan* pl, bool xp) {
     const int n_sms = n_sms_current();
     const double out_bytes_per_col = 128.0 * ((d->out0 ? pl->esize : 0) + (d->out1_mode == OCCD_OUT1_CL ? pl->esize : 0) +
                                               (d->out1_mode == OCCD_OUT1_F32_PLANAR ? 4 : 0));
-    // experiment hook (tools/conv_bench.py, bench.py): OCCD_EPI_RATE overrides the model's epilogue drain rate
-    static const double epi_rate = [] { const char* e = getenv("OCCD_EPI_RATE"); const double v = e ? atof(e) : 0.0;
-                                        return v > 0.0 ? v : 12.0; }();
+    const double epi_rate = 12.0;
     double best = -1.0;
     t.N_tile = 16;
     for (int n = 16; n <= 256 && n <= d->Cout_pad; n += 16) {
@@ -1466,7 +1349,6 @@ static int tc_geometry(const occd_conv_desc* d, occd_conv_plan* pl, bool xp) {
   while (t.tmem_cols < t.N_tile) t.tmem_cols *= 2;
   t.trace = g_trace_buf;
   t.tmem_cols *= 2;  // two accumulators: the epilogue of tile j overlaps the MMAs of tile j+1
-  t.pdl = pdl_enabled();
   t.a_bytes = 128 * RB;
   t.b_bytes = t.N_tile * RB;
   t.b_stride = round_up(t.b_bytes, 1024);
@@ -1501,65 +1383,39 @@ static int tc_geometry(const occd_conv_desc* d, occd_conv_plan* pl, bool xp) {
   t.stages = stages;
   pl->smem = (size_t)stages * group * stage_bytes + 16 * kMaxStages + 64 + 1024;  // + barriers + alignment slack
   const long long m_tiles = (long long)d->B * t.tiles_d * t.tiles_h * t.tiles_w;
-  const long long all_tiles = m_tiles * (xp ? 1 : d->Cout_pad / t.N_tile) * n_groups;
-  if (all_tiles > 2147483647LL) {
-    occd_set_last_error("occd_conv_plan_create: too many tiles");
-    return OCCD_ERR_UNSUPPORTED;
-  }
+  const int rg = persistent_grid(pl, m_tiles * (xp ? 1 : d->Cout_pad / t.N_tile) * n_groups);
+  if (rg != OCCD_OK) return rg;
   t.num_m_tiles = (int)m_tiles;
-  {
-    const int n_sms = n_sms_current();
-    pl->grid = dim3((unsigned)(all_tiles < n_sms ? all_tiles : n_sms));
-  }
-  return OCCD_OK;
+  const int box[3] = {t.TW * d->stride[2], t.TH * d->stride[1], t.TD * d->stride[0]};
+  const int estr[3] = {d->stride[2], d->stride[1], d->stride[0]};
+  return encode_maps(d, pl, box, estr, t.N_tile);
 }
 
-static int tc_encode(const occd_conv_desc* d, occd_conv_plan* pl) {
-  const TcParams& t = pl->tc;
-  const int KC = pl->kc, es = pl->esize;
-  EncodeTiledFn enc = get_encode_fn();
-  if (!enc) {
-    occd_set_last_error("occd_conv_plan_create: cuTensorMapEncodeTiled unavailable (no CUDA driver / GPU?)");
-    return OCCD_ERR_CUDA;
+// Hands the kernel instantiation of a tcgen05 plan (dtype x impl x K-chunk row bytes) and its arguments to
+// f(kernel, args...)
+template <typename T, int RB, typename F>
+static cudaError_t with_tc_kernel_rb(const occd_conv_plan* pl, F&& f) {
+  switch (pl->impl) {
+    case OCCD_CONV_IMPL_TC: return f(conv_tc_kernel<T, RB, false>, pl->tc, pl->tmA[0], pl->tmA[1], pl->tmA[2], pl->tmW);
+    case OCCD_CONV_IMPL_TCX: return f(conv_tc_kernel<T, RB, true>, pl->tc, pl->tmA[0], pl->tmA[1], pl->tmA[2], pl->tmW);
+    case OCCD_CONV_IMPL_HALO: return f(conv_halo_kernel<T, RB>, pl->halo, pl->tmA[0], pl->tmW);
+    default: return f(conv_halox_kernel<T, RB>, pl->halox, pl->tmA[0], pl->tmW);
   }
-  const CUtensorMapSwizzle sw = swizzle_for(pl->rb);
-  for (int s = 0; s < d->n_src; ++s) {
-    const cuuint64_t cs = (cuuint64_t)d->src_cstride[s] * es;
-    cuuint64_t gdim[5] = {(cuuint64_t)d->src_C[s], (cuuint64_t)d->IW, (cuuint64_t)d->IH, (cuuint64_t)d->ID,
-                          (cuuint64_t)d->B};
-    cuuint64_t gstr[4] = {cs, cs * d->IW, cs * d->IW * d->IH, cs * d->IW * d->IH * d->ID};
-    cuuint32_t box[5] = {(cuuint32_t)KC, (cuuint32_t)(t.TW * d->stride[2]), (cuuint32_t)(t.TH * d->stride[1]),
-                         (cuuint32_t)(t.TD * d->stride[0]), 1};
-    cuuint32_t estr[5] = {1, (cuuint32_t)d->stride[2], (cuuint32_t)d->stride[1], (cuuint32_t)d->stride[0], 1};
-    void* base = (void*)((const char*)d->src[s] + (size_t)d->src_coff[s] * es);
-    CUresult r = enc(&pl->tmA[s], tm_dtype(pl->dtype), 5, base, gdim, gstr, box, estr,
-                     CU_TENSOR_MAP_INTERLEAVE_NONE, sw, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-      char msg[160];
-      snprintf(msg, sizeof(msg), "occd_conv_plan_create: cuTensorMapEncodeTiled(source %d) failed with %d", s, (int)r);
-      occd_set_last_error(msg);
-      return OCCD_ERR_CUDA;
-    }
+}
+
+template <typename T, typename F>
+static cudaError_t with_tc_kernel_t(const occd_conv_plan* pl, F&& f) {
+  switch (pl->rb) {
+    case 128: return with_tc_kernel_rb<T, 128>(pl, f);
+    case 64: return with_tc_kernel_rb<T, 64>(pl, f);
+    default: return with_tc_kernel_rb<T, 32>(pl, f);
   }
-  for (int s = d->n_src; s < OCCD_CONV_MAX_SRC; ++s) pl->tmA[s] = pl->tmA[0];
-  {
-    cuuint64_t gdim[2] = {(cuuint64_t)d->Kpad,
-                          (cuuint64_t)d->n_taps * d->Cout_pad * (d->weight_per_image ? d->B : 1)};
-    cuuint64_t gstr[1] = {(cuuint64_t)d->Kpad * es};
-    cuuint32_t box[2] = {(cuuint32_t)KC, (cuuint32_t)t.N_tile};
-    cuuint32_t estr[2] = {1, 1};
-    CUresult r = enc(&pl->tmW, tm_dtype(pl->dtype), 2, (void*)d->weight, gdim, gstr, box, estr,
-                     CU_TENSOR_MAP_INTERLEAVE_NONE, sw, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-      char msg[160];
-      snprintf(msg, sizeof(msg), "occd_conv_plan_create: cuTensorMapEncodeTiled(weights) failed with %d", (int)r);
-      occd_set_last_error(msg);
-      return OCCD_ERR_CUDA;
-    }
-  }
-  return OCCD_OK;
+}
+
+template <typename F>
+static cudaError_t with_tc_kernel(const occd_conv_plan* pl, F&& f) {
+  if (pl->dtype == OCCD_DTYPE_F32) return with_tc_kernel_t<float>(pl, f);
+  return with_tc_kernel_t<__nv_bfloat16>(pl, f);
 }
 
 extern "C" int occd_conv_plan_create(const occd_conv_desc* d, occd_conv_plan** out) {
@@ -1641,16 +1497,18 @@ extern "C" int occd_conv_plan_create(const occd_conv_desc* d, occd_conv_plan** o
     return OCCD_OK;
   }
 
-  int rc;
-  if (d->impl == OCCD_CONV_IMPL_HALO) {
-    rc = halo_geometry(d, pl);
-    if (rc == OCCD_OK) rc = halo_encode(d, pl);
-  } else if (d->impl == OCCD_CONV_IMPL_HALOX) {
-    rc = halox_geometry(d, pl);
-    if (rc == OCCD_OK) rc = halox_encode(d, pl);
-  } else {
-    rc = tc_geometry(d, pl, d->impl == OCCD_CONV_IMPL_TCX);
-    if (rc == OCCD_OK) rc = tc_encode(d, pl);
+  int rc = d->impl == OCCD_CONV_IMPL_HALO    ? plan_halo(d, pl)
+           : d->impl == OCCD_CONV_IMPL_HALOX ? plan_halox(d, pl)
+                                             : plan_tc(d, pl, d->impl == OCCD_CONV_IMPL_TCX);
+  if (rc == OCCD_OK) {
+    // the plan's pointers belong to the device current at creation: its kernel may use up to 227 KB of smem there
+    const cudaError_t e = with_tc_kernel(pl, [](auto kernel, const auto&...) {
+      return cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+    });
+    if (e != cudaSuccess) {
+      occd_set_last_error(cudaGetErrorString(e));
+      rc = OCCD_ERR_CUDA;
+    }
   }
   if (rc != OCCD_OK) { delete pl; return rc; }
   *out = pl;
@@ -1689,114 +1547,24 @@ extern "C" int occd_conv_plan_info(const occd_conv_plan* pl, int* info) {
   return OCCD_OK;
 }
 
-template <typename T, int RB, bool XP>
-static int launch_tc(const occd_conv_plan* pl, cudaStream_t st) {
-  static bool attr_set[64] = {false};  // per instantiation, per device (the attribute is per device)
-  int dev = 0;
-  cudaGetDevice(&dev);
-  if (dev < 0 || dev >= 64) dev = 0;
-  if (!attr_set[dev]) {
-    cudaError_t e = cudaFuncSetAttribute(conv_tc_kernel<T, RB, XP>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-    if (e != cudaSuccess) { occd_set_last_error(cudaGetErrorString(e)); return OCCD_ERR_CUDA; }
-    attr_set[dev] = true;
-  }
-  if (pl->tc.pdl) {
-    cudaError_t e = launch_pdl(conv_tc_kernel<T, RB, XP>, pl->grid, kTcThreads, pl->smem, st, pl->tc, pl->tmA[0],
-                               pl->tmA[1], pl->tmA[2], pl->tmW);
-    if (e != cudaSuccess) { occd_set_last_error(cudaGetErrorString(e)); return OCCD_ERR_CUDA; }
-    return OCCD_OK;
-  }
-  conv_tc_kernel<T, RB, XP><<<pl->grid, kTcThreads, pl->smem, st>>>(pl->tc, pl->tmA[0], pl->tmA[1], pl->tmA[2], pl->tmW);
-  OCCD_CHECK_LAUNCH();
-  return OCCD_OK;
-}
-
-template <typename T, int RB>
-static int launch_halo(const occd_conv_plan* pl, cudaStream_t st) {
-  static bool attr_set[64] = {false};  // per device
-  int dev = 0;
-  cudaGetDevice(&dev);
-  if (dev < 0 || dev >= 64) dev = 0;
-  if (!attr_set[dev]) {
-    cudaError_t e = cudaFuncSetAttribute(conv_halo_kernel<T, RB>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-    if (e != cudaSuccess) { occd_set_last_error(cudaGetErrorString(e)); return OCCD_ERR_CUDA; }
-    attr_set[dev] = true;
-  }
-  if (pl->halo.pdl) {
-    cudaError_t e = launch_pdl(conv_halo_kernel<T, RB>, pl->grid, kTcThreads, pl->smem, st, pl->halo, pl->tmA[0],
-                               pl->tmW);
-    if (e != cudaSuccess) { occd_set_last_error(cudaGetErrorString(e)); return OCCD_ERR_CUDA; }
-    return OCCD_OK;
-  }
-  conv_halo_kernel<T, RB><<<pl->grid, kTcThreads, pl->smem, st>>>(pl->halo, pl->tmA[0], pl->tmW);
-  OCCD_CHECK_LAUNCH();
-  return OCCD_OK;
-}
-
-template <typename T, int RB>
-static int launch_halox(const occd_conv_plan* pl, cudaStream_t st) {
-  static bool attr_set[64] = {false};  // per device
-  int dev = 0;
-  cudaGetDevice(&dev);
-  if (dev < 0 || dev >= 64) dev = 0;
-  if (!attr_set[dev]) {
-    cudaError_t e = cudaFuncSetAttribute(conv_halox_kernel<T, RB>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-    if (e != cudaSuccess) { occd_set_last_error(cudaGetErrorString(e)); return OCCD_ERR_CUDA; }
-    attr_set[dev] = true;
-  }
-  if (pl->halox.pdl) {
-    cudaError_t e = launch_pdl(conv_halox_kernel<T, RB>, pl->grid, kTcThreads, pl->smem, st, pl->halox, pl->tmA[0],
-                               pl->tmW);
-    if (e != cudaSuccess) { occd_set_last_error(cudaGetErrorString(e)); return OCCD_ERR_CUDA; }
-    return OCCD_OK;
-  }
-  conv_halox_kernel<T, RB><<<pl->grid, kTcThreads, pl->smem, st>>>(pl->halox, pl->tmA[0], pl->tmW);
-  OCCD_CHECK_LAUNCH();
-  return OCCD_OK;
-}
-
-template <typename T>
-static int run_typed(const occd_conv_plan* pl, cudaStream_t st) {
-  if (pl->impl == OCCD_CONV_IMPL_SIMT) {
-    conv_simt_kernel<T><<<pl->grid, 128, 0, st>>>(pl->simt);
-    OCCD_CHECK_LAUNCH();
-    return OCCD_OK;
-  }
-  if (pl->impl == OCCD_CONV_IMPL_HALO) {
-    switch (pl->rb) {
-      case 128: return launch_halo<T, 128>(pl, st);
-      case 64: return launch_halo<T, 64>(pl, st);
-      case 32: return launch_halo<T, 32>(pl, st);
-    }
-  }
-  if (pl->impl == OCCD_CONV_IMPL_HALOX) {
-    switch (pl->rb) {
-      case 128: return launch_halox<T, 128>(pl, st);
-      case 64: return launch_halox<T, 64>(pl, st);
-      case 32: return launch_halox<T, 32>(pl, st);
-    }
-  }
-  if (pl->impl == OCCD_CONV_IMPL_TCX) {
-    switch (pl->rb) {
-      case 128: return launch_tc<T, 128, true>(pl, st);
-      case 64: return launch_tc<T, 64, true>(pl, st);
-      case 32: return launch_tc<T, 32, true>(pl, st);
-    }
-  }
-  if (pl->impl == OCCD_CONV_IMPL_TC) {
-    switch (pl->rb) {
-      case 128: return launch_tc<T, 128, false>(pl, st);
-      case 64: return launch_tc<T, 64, false>(pl, st);
-      case 32: return launch_tc<T, 32, false>(pl, st);
-    }
-  }
-  occd_set_last_error("occd_conv_run: bad plan");
-  return OCCD_ERR_ARG;
-}
-
 extern "C" int occd_conv_run(const occd_conv_plan* pl, void* stream) {
   OCCD_CHECK_ARG(pl != nullptr, "occd_conv_run: null plan");
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  if (pl->dtype == OCCD_DTYPE_F32) return run_typed<float>(pl, st);
-  return run_typed<__nv_bfloat16>(pl, st);
+  if (pl->impl == OCCD_CONV_IMPL_SIMT) {
+    if (pl->dtype == OCCD_DTYPE_F32) conv_simt_kernel<float><<<pl->grid, 128, 0, st>>>(pl->simt);
+    else conv_simt_kernel<__nv_bfloat16><<<pl->grid, 128, 0, st>>>(pl->simt);
+    OCCD_CHECK_LAUNCH();
+    return OCCD_OK;
+  }
+  // programmatic dependent launch (common.cuh): the prologue of the persistent kernels overlaps the tail of the
+  // previous grid.  Measured on B200 (round 2, profiles/r02_ab_experiments.txt): 1.0 % of the config-2 forward,
+  // results bit-identical.
+  const cudaError_t e = with_tc_kernel(pl, [&](auto kernel, const auto&... args) {
+    return occd_launch(kernel, pl->grid, dim3(kTcThreads), pl->smem, st, args...);
+  });
+  if (e != cudaSuccess) {
+    occd_set_last_error(cudaGetErrorString(e));
+    return OCCD_ERR_CUDA;
+  }
+  return OCCD_OK;
 }

@@ -22,8 +22,6 @@ struct ConvEpi {
   int out1_mode;
   void* out1;
   int out1_cstride, out1_coff, out1_C;
-  int dbg;   // experiment switch (OCCD_DEBUG_EPI, tools/conv_bench.py only): 1 = skip the out0 stores, 2 = skip the
-             // whole row epilogue (TMEM drain only)
 };
 
 __device__ __forceinline__ long long epi_pos(const ConvEpi& e, int b, int od, int oh, int ow, int oa0, int oa1,
@@ -89,17 +87,9 @@ __device__ __forceinline__ void conv_epilogue_compute(const ConvEpi& e, long lon
 template <typename T, int NV>
 __device__ __forceinline__ void conv_epilogue_row(const ConvEpi& e, int b, int od, int oh, int ow, int n0,
                                                   float* v) {
-  if (e.dbg == 2) return;
   const long long pos = epi_pos(e, b, od, oh, ow);
   conv_epilogue_compute<T, NV>(e, pos, b, n0, v);
   if (!e.out0) return;
-  if (e.dbg == 1) {   // keep the arithmetic alive without storing
-    float s = 0.f;
-#pragma unroll
-    for (int i = 0; i < NV; ++i) s += v[i];
-    if (s == 123456.789f) reinterpret_cast<T*>(e.out0)[0] = Elem<T>::cvt(s);
-    return;
-  }
 #pragma unroll
   for (int g = 0; g < NV; g += 8) {
     const int n = n0 + g;
@@ -113,7 +103,7 @@ __device__ __forceinline__ void conv_epilogue_row(const ConvEpi& e, int b, int o
 
 // ---------------------------------------------------------------------------------------------------------------
 // Fast path of the per-tap and halo kernels' epilogue (out0 only: no second output, no post-activation residual).  Measured
-// on B200 (tools/conv_bench.py with OCCD_DEBUG_EPI, round 2): the row epilogue above is LATENCY bound -- 4 epilogue
+// on B200 (round 2, profiles/r02_lift_variants.txt): the row epilogue above is LATENCY bound -- 4 epilogue
 // warps per scheduler walk a serial chain tcgen05.ld -> wait -> bias loads -> (residual loads) -> math -> store per
 // 16 columns, at ~15 % of the SM's issue rate.  Here the chunk's bias (and residual) loads are issued BEFORE the wait
 // on its TMEM load, the output / residual row pointers are formed once per tile, and the activation switch runs once
@@ -214,7 +204,7 @@ __device__ __forceinline__ void epi_finish(const EpiRow<T>& e, int c0, const uin
 
 // out0 only, and at most one residual: res1 (before the activation) or a post-activation res2
 __device__ __forceinline__ bool epi_fast_ok(const ConvEpi& e) {
-  return e.out1_mode == OCCD_OUT1_NONE && e.out0 != nullptr && e.dbg <= 1 &&
+  return e.out1_mode == OCCD_OUT1_NONE && e.out0 != nullptr &&
          (e.res2 == nullptr || (e.res2_post && e.res1 == nullptr));
 }
 
@@ -225,7 +215,7 @@ __device__ __forceinline__ EpiRow<T> epi_row(const ConvEpi& e, bool valid, int b
                                              int oa0, int oa1, int oa2) {
   EpiRow<T> er;
   const long long pos = valid ? epi_pos(e, b, od, oh, ow, oa0, oa1, oa2) : 0;
-  er.out = (valid && e.dbg == 0) ? reinterpret_cast<T*>(e.out0) + pos * e.out0_cstride + e.out0_coff + n0 : nullptr;
+  er.out = valid ? reinterpret_cast<T*>(e.out0) + pos * e.out0_cstride + e.out0_coff + n0 : nullptr;
   er.res = nullptr;
   er.res_post = 0;
   if (valid && e.res1) {

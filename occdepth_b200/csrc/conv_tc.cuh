@@ -8,28 +8,12 @@ namespace tc {
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
-__device__ __forceinline__ bool elect_one() {
-  uint32_t pred = 0;
-  asm volatile(
-      "{\n"
-      ".reg .b32 rx;\n"
-      ".reg .pred px;\n"
-      "elect.sync rx|px, 0xffffffff;\n"
-      "selp.b32 %0, 1, 0, px;\n"
-      "}\n"
-      : "=r"(pred));
-  return pred != 0;
-}
-
 // ---------------- mbarrier ----------------
 __device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
   asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
 }
 __device__ __forceinline__ void fence_barrier_init() {
   asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-}
-__device__ __forceinline__ void fence_proxy_async() {
-  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
 }
 __device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
   asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
@@ -104,17 +88,6 @@ __device__ __forceinline__ uint64_t make_sdesc(uint32_t saddr, uint32_t row_byte
   return d;
 }
 
-// descriptor for a start address that is NOT aligned to the swizzle repeat (8 rows): bits [49,52) "base offset"
-// would tell the hardware where in the 8-row pattern the first row sits.  Measured on B200 (tools/gpu_diag.py halo):
-// with TMA-written tiles whose stage base is 1024-byte aligned the XOR swizzle is a function of the ABSOLUTE shared
-// address bits on both the TMA and the UMMA side, so a row-shifted start address needs base offset 0 (mode 0,
-// bit-exact); mode 1 = (addr >> 7) & 7 produced wrong results and is kept only for experiments.
-__device__ __forceinline__ uint64_t make_sdesc_shifted(uint32_t saddr, uint32_t row_bytes, int mode) {
-  uint64_t d = make_sdesc(saddr, row_bytes);
-  if (mode == 1) d |= (uint64_t)((saddr >> 7) & 7u) << 49;
-  return d;
-}
-
 // instruction descriptor, both operands K-major, F32 accumulate
 //   bits [4,6) D format (1 = F32)  [7,10) A format  [10,13) B format  [15] A major  [16] B major
 //   bits [17,23) N >> 3            [24,29) M >> 4
@@ -126,19 +99,7 @@ __host__ __device__ constexpr uint32_t make_idesc_tf32(int M, int N) {
   return (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
 }
 
-__device__ __forceinline__ void mma_bf16(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
-                                         uint32_t accumulate) {
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "setp.ne.b32 p, %4, 0;\n"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n"
-      "}\n" ::"r"(tmem_d),
-      "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-
-// same, with the accumulate flag as an immediate (no per-instruction setp in the issue loop)
+// kind::f16 (BF16 operands); the accumulate flag is an immediate (no per-instruction setp in the issue loop)
 template <int ACC>
 __device__ __forceinline__ void mma_bf16_imm(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc) {
   asm volatile(
@@ -181,6 +142,16 @@ template <> struct Mma<float> {
     mma_tf32_imm<ACC>(d, a, b, id);
   }
 };
+
+// one K chunk: NMMA instructions over consecutive 32-byte slices of the A / B rows (descriptor address units of 16
+// bytes); `first` starts the accumulator with the chunk's first instruction instead of adding to it
+template <typename T, int NMMA>
+__device__ __forceinline__ void mma_kchunk(uint32_t d, uint64_t da, uint64_t db, uint32_t idesc, bool first) {
+  if (first) Mma<T>::template issue<0>(d, da, db, idesc);
+  else Mma<T>::template issue<1>(d, da, db, idesc);
+#pragma unroll
+  for (int k = 1; k < NMMA; ++k) Mma<T>::template issue<1>(d, da + 2 * k, db + 2 * k, idesc);
+}
 
 // arrive on an mbarrier when all previously issued tcgen05.mma of this thread have completed
 __device__ __forceinline__ void mma_commit(uint32_t bar) {

@@ -69,7 +69,7 @@ def default_impl():
 
 
 def halox_eligible(srcs, taps, stride, omul, out_dims, Cout_pad, weight_buf):
-    """shape test mirroring halox_geometry (csrc/conv.cu): stride-1 'same' conv on a grid whose innermost extent W is
+    """shape test mirroring plan_halox (csrc/conv.cu): stride-1 'same' conv on a grid whose innermost extent W is
     8 / 16 / 32, taps = (dz, dy) groups of dx = -d, 0, +d with dz, dy in {-d, 0, d}, one K chunk, 3*Cout_pad <= 256"""
     if len(srcs) != 1 or weight_buf is not None or len(taps) % 3 or not 3 <= len(taps) <= 27:
         return False
@@ -103,7 +103,7 @@ def tcx_eligible(taps, stride, Cout_pad):
 
 
 def halo_eligible(srcs, taps, stride, omul, out_dims, Cout_pad, weight_buf):
-    """shape test mirroring halo_geometry (csrc/conv.cu): stride-1 'same' conv, {-d,0,d} taps, one K chunk"""
+    """shape test mirroring plan_halo (csrc/conv.cu): stride-1 'same' conv, {-d,0,d} taps, one K chunk"""
     if len(srcs) != 1 or weight_buf is not None or len(taps) < 3 or len(taps) > 27:
         return False
     if tuple(stride) != (1, 1, 1) or tuple(omul) != (1, 1, 1) or tuple(out_dims) != tuple(srcs[0].dims[1:]):
@@ -276,18 +276,21 @@ class ConvOp:
         d = _lib.ConvDesc()
         if impl is None:
             impl = default_impl()
-        auto = impl is None
         if groups:
-            auto, impl = False, _lib.CONV_IMPL_TC
-        if auto:
-            impl = (_lib.CONV_IMPL_HALO if halo_eligible(srcs, taps, stride, omul, out_dims, Cout_pad, weight_buf)
-                    else _lib.CONV_IMPL_TC)
-            if impl == _lib.CONV_IMPL_TC and tcx_eligible(taps, stride, Cout_pad):
-                impl = _lib.CONV_IMPL_TCX
+            impls = [_lib.CONV_IMPL_TC]
+        elif impl is not None:
+            impls = [impl]
+        else:
+            # auto: the candidates in order of preference, each tried until occd_conv_plan_create accepts one (its
+            # geometry may still decline, e.g. when the weights and one stage do not fit in shared memory)
+            impls = []
             if halox_eligible(srcs, taps, stride, omul, out_dims, Cout_pad, weight_buf):
-                self._fallback = impl
-                impl = _lib.CONV_IMPL_HALOX
-        d.impl = impl
+                impls.append(_lib.CONV_IMPL_HALOX)
+            if halo_eligible(srcs, taps, stride, omul, out_dims, Cout_pad, weight_buf):
+                impls.append(_lib.CONV_IMPL_HALO)
+            elif tcx_eligible(taps, stride, Cout_pad):
+                impls.append(_lib.CONV_IMPL_TCX)
+            impls.append(_lib.CONV_IMPL_TC)
         d.dtype = LIB_DTYPE[precision_of(adt)]
         d.n_src = len(srcs)
         for i, s in enumerate(srcs):
@@ -339,16 +342,11 @@ class ConvOp:
         self.desc = d
         self.flops = 2 * B * OD * OH * OW * Cout * sum(srcs[t[0]].C for t in taps)
         h = C.c_void_p()
-        rc = _lib.lib().occd_conv_plan_create(C.byref(d), C.byref(h))
-        if rc != 0 and auto and d.impl == _lib.CONV_IMPL_HALOX:
-            d.impl = self._fallback         # geometry declined (e.g. weights + one stage do not fit)
+        for impl in impls:
+            d.impl = impl
             rc = _lib.lib().occd_conv_plan_create(C.byref(d), C.byref(h))
-        if rc != 0 and auto and d.impl == _lib.CONV_IMPL_TCX:
-            d.impl = _lib.CONV_IMPL_TC
-            rc = _lib.lib().occd_conv_plan_create(C.byref(d), C.byref(h))
-        if rc != 0 and auto and d.impl == _lib.CONV_IMPL_HALO:
-            d.impl = _lib.CONV_IMPL_TC      # shape did not fit the halo scheme: per-tap tcgen05 kernel
-            rc = _lib.lib().occd_conv_plan_create(C.byref(d), C.byref(h))
+            if rc == 0:
+                break
         _lib.check(rc, "occd_conv_plan_create(%s)" % name)
         self.handle = h
         self.impl = d.impl

@@ -31,5 +31,4 @@ t0 = int(t[0, 0])
 print(n, plan.ops[0].info())
 print("tile: prod_start prod_end | mma_start mma_end | epi_wait epi_go epi_end   (cycles since first stamp)")
 for j in range(12):
-    x = int(t[j, 7])
-    print(j, [int(v) - t0 if v else None for v in t[j, :7]], "ld-wait %d, row-epilogue %d cycles (first half-chunks only)" % (x >> 32, x & 0xffffffff) if x else "")
+    print(j, [int(v) - t0 if v else None for v in t[j, :7]])
