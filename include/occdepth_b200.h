@@ -54,9 +54,13 @@ typedef struct {
   long long vstride[OCCD_SFA_MAX_SCALES]; /* elements between consecutive views; 0 = dense (h*w*C)    */
   int n_scales;                 /* 1..4                                                            */
   int n_views;                  /* V, 1..4                                                         */
-  int C;                        /* channels, multiple of 4 (f32) / 8 (bf16), <= 256                */
+  int C;                        /* channels, multiple of 4 (f32) / 8 (bf16), <= 256 (f32) / 512 (bf16) */
   int feat_dtype;               /* OCCD_DTYPE_*                                                    */
   const int64_t* pix;           /* [V][N][P][2] (x,y) int64 -- batch["projected_pix_s"][i]         */
+                                /* a point with fov set whose flat index (y//div)*w + (x//div) lies */
+                                /* outside [0, h*w) gathers zeros but still counts toward the mean  */
+                                /* over the pattern and toward the view mask (the reference leaves  */
+                                /* this case undefined: its gather raises or wraps)                 */
   const uint8_t* fov;           /* [V][N][P] bool          -- batch["fov_mask_s"][i]               */
   long long N;                  /* voxels                                                          */
   int P;                        /* pattern points per voxel (1 for pattern_id 0)                   */
@@ -72,7 +76,8 @@ typedef struct {
 int occd_sfa_lift_fwd(const occd_sfa_params* p, void* stream);
 
 /* layout helpers at the module boundary: NCHW/NCDHW fp32 <-> channels-last (f32 or bf16)          */
-/* in: [B][C][S] planar fp32, out: [B][S][cstride] channels-last (pad channels zero-filled)        */
+/* in: [B][C][S] planar fp32, out: [B][S][cstride] channels-last (pad channels zero-filled), every */
+/* value rounded to out_dtype: bf16 round-to-nearest-even, or TF32 for OCCD_DTYPE_F32              */
 int occd_planar_to_cl(const float* in, void* out, int out_dtype, long long B, int C, long long S,
                       int cstride, void* stream);
 /* in: [B][S][cstride] channels-last, out: [B][C][S] planar fp32                                   */

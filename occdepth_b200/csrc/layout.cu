@@ -37,7 +37,7 @@ __global__ void planar_to_cl_kernel(const float* __restrict__ in, OT* __restrict
     if (s < S && c < cstride) {
       const float v = tile[threadIdx.x][i];
       if constexpr (sizeof(OT) == 2) outb[s * cstride + c] = __float2bfloat16_rn(v);
-      else outb[s * cstride + c] = v;
+      else outb[s * cstride + c] = round_tf32(v);   // OCCD_DTYPE_F32 buffers hold TF32 values (kind::tf32 operands)
     }
   }
 }

@@ -48,12 +48,11 @@ class SFA(nn.Module):
             raise RuntimeError("SFA: channel count must be a multiple of 4")
         pix = projected_pix.to(device=dev, dtype=torch.int64).contiguous()
         fov = fov_mask.to(device=dev, dtype=torch.bool).contiguous()
-        # NCHW fp32 -> channels-last fp32 (the kernel gathers one contiguous C-vector per pixel)
-        feat = torch.empty(n_views, h * w, c, dtype=torch.float32, device=dev)
+        # NCHW fp32 -> channels-last fp32 (the kernel gathers one contiguous C-vector per pixel).  A plain copy, not
+        # occd_planar_to_cl: that one rounds to TF32, and this module returns the reference's exact fp32 lift
+        feat = x2d.float().permute(0, 2, 3, 1).contiguous()
         L = _lib.lib()
         st = _lib.stream_ptr()
-        _lib.check(L.occd_planar_to_cl(x2d.contiguous().float().data_ptr(), feat.data_ptr(), _lib.DTYPE_F32,
-                                       n_views, c, h * w, c, st), "occd_planar_to_cl")
         S = [s // self.project_scale for s in self.scene_size]
         N = pix.shape[1]
         if N != S[0] * S[1] * S[2]:

@@ -419,11 +419,12 @@ def depth_net(sd, p, x, cam_k4):
 def frustum_grid(grid_size, pc_min, pc_max, lidar_to_cam, cam_k4, ida, image_hw, num_bins, dmin, dmax):
     """frustum_grid_generator.py:20-152 for one camera: -> (1, X, Y, Z, 3) normalised sampling grid."""
     X, Y, Z = grid_size
-    vs = (pc_max - pc_min) / torch.tensor([X, Y, Z], dtype=torch.float32)
-    i, j, k = torch.meshgrid(torch.arange(X, dtype=torch.float32), torch.arange(Y, dtype=torch.float32),
-                             torch.arange(Z, dtype=torch.float32), indexing="ij")
+    dt = lidar_to_cam.dtype                      # float32 as in the reference; float64 for kernel-level tests
+    vs = (pc_max - pc_min) / torch.tensor([X, Y, Z], dtype=dt)
+    i, j, k = torch.meshgrid(torch.arange(X, dtype=dt), torch.arange(Y, dtype=dt),
+                             torch.arange(Z, dtype=dt), indexing="ij")
     vox = torch.stack([i, j, k], -1) + 0.5                                       # :31-42
-    G = torch.eye(4)
+    G = torch.eye(4, dtype=dt)
     G[0, 0], G[1, 1], G[2, 2] = vs
     G[:3, 3] = pc_min
     trans = lidar_to_cam @ G                                                     # :95
@@ -441,7 +442,7 @@ def frustum_grid(grid_size, pc_min, pc_max, lidar_to_cam, cam_k4, ida, image_hw,
     fh = F.pad(fg, [0, 1], value=1.0) @ ida.t()                                   # :113-114
     w = fh[..., 3:]
     fg = fh[..., :3] * torch.where(w.abs() > 1e-8, 1.0 / (w + 1e-8), torch.ones_like(w))
-    shape = torch.tensor([float(image_hw[1]), float(image_hw[0]), float(num_bins)])   # flipped [D,H,W], :139-145
+    shape = torch.tensor([float(image_hw[1]), float(image_hw[0]), float(num_bins)], dtype=dt)   # flipped [D,H,W], :139-145
     fg = fg / (shape - 1) * 2 - 1
     fg[~torch.isfinite(fg)] = -2                                                  # :148-150
     return fg.unsqueeze(0)
